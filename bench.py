@@ -168,6 +168,8 @@ def main():
   ap.add_argument('--no-steady', action='store_true', help='skip the attached steady-state (cycling episodes) measurement')
   ap.add_argument('--steady-steps', type=int, default=200)
   ap.add_argument('--steady-warmup', type=int, default=100)
+  ap.add_argument('--dump-outputs', metavar='DIR', help='write the TimeStep of the last timed step of the headline workload (rank 0) '
+                                                        'to DIR/<name>.npy, float32; see dump_outputs()')
   a = ap.parse_args()
   global PROFILER_RANGE
   PROFILER_RANGE = bool(a.profiler_range)
@@ -208,7 +210,7 @@ def main():
   dev = torch.device('cuda', local_rank)
   if world > 1:
     dist.init_process_group('nccl', device_id=dev)
-  res = run_workload(a.workload, envs, a.steps, a.warmup, a.precision, dev, rank, world, local_rank)
+  res = run_workload(a.workload, envs, a.steps, a.warmup, a.precision, dev, rank, world, local_rank, dump_dir=a.dump_outputs)
   if rank == 0:
     out = dict(metric=METRIC, value=res['value'], unit='env-steps/s', n_gpus=world, steps=a.steps, warmup=a.warmup,
                ms_per_step=res['ms_per_step'], higher_is_better=True, scaling='weak', vs_baseline=None,
@@ -257,9 +259,32 @@ def _actions(env, n, envs, dev, seed):
 
 
 PROFILER_RANGE = False   # set by --profiler-range
+DUMP_MAX_BYTES = 64 * 10**6   # --dump-outputs: .npy headers included
 
 
-def run_workload(name, envs, steps, warmup, precision, dev, rank, world, local_rank):
+def dump_outputs(out_dir, ts, max_bytes=DUMP_MAX_BYTES):
+  """Writes what a caller of env.step() receives - step_type, reward, discount and every non-empty observation - as
+  out_dir/<name>.npy in float32, one row per env.  If that exceeds `max_bytes`, a fixed sample of envs (seed 0, sorted, the
+  same rows in every file) is written instead, with its env indices in env_index.npy (float64).  Returns the file names.
+  With the same arguments the rows repeat bit for bit from run to run, except those of envs that lost contacts to a full per-env
+  buffer (BatchedEnvironment.contacts_dropped_per_env): which contacts such an env keeps depends on the order they arrive in."""
+  arrays = dict(step_type=ts.step_type, reward=ts.reward, discount=ts.discount, **{k: v for k, v in ts.observation.items() if v.numel()})
+  arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+  n = len(arrays['reward'])
+  header = 128   # bytes of one .npy header for these shapes
+  if sum(a.nbytes + header for a in arrays.values()) > max_bytes:
+    per_env = sum(a[0].nbytes for a in arrays.values()) + 8
+    k = (max_bytes - header * (len(arrays) + 1)) // per_env
+    idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    arrays = {name: a[idx] for name, a in arrays.items()}
+    arrays['env_index'] = idx.astype(np.float64)
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), a)
+  return sorted(name + '.npy' for name in arrays)
+
+
+def run_workload(name, envs, steps, warmup, precision, dev, rank, world, local_rank, dump_dir=None):
   import torch
   import torch.distributed as dist
   from so101_sim_b200.sharding import EpisodeStats, gather_episode_stats, rank_seed
@@ -314,6 +339,8 @@ def run_workload(name, envs, steps, warmup, precision, dev, rank, world, local_r
     t_wall = time.perf_counter() - t_wall0
   if PROFILER_RANGE:
     torch.cuda.synchronize(); torch.cuda.profiler.stop()
+  if dump_dir and rank == 0:   # before the passes below step the env again and overwrite the TimeStep's buffers
+    dump_outputs(dump_dir, ts)
   c1 = env.counters()
   drop_names = ('per_pair', 'candidates', 'pairs', 'queue', 'raw_contacts', 'jacobian_blocks', 'hits')
   drops = dict(zip(drop_names, [int(x) for x in env.debug_read('dropcat', 8)[0, :7].tolist()])) if w['collide'] and envs >= 8 else {}

@@ -108,6 +108,35 @@ def test_bench_reference_arm_prints_the_contract_line():
   assert d['vs_baseline'] is None and d['steps'] == 1 and d['warmup'] == 0
 
 
+def test_bench_dump_outputs_writes_the_timestep(tmp_path):
+  """bench.py --dump-outputs: every non-empty block of the TimeStep as float32 <name>.npy, one row per env; above the byte budget
+  the same fixed sample of rows in every file, their env indices beside them, and the whole dump within the budget."""
+  import torch
+  import bench
+  from so101_sim_b200.task_suite import OBSERVATION_KEYS, BatchedTimeStep
+  N = 1000
+  g = torch.Generator().manual_seed(0)
+  obs = {k: torch.zeros(N, 0) if k.endswith('joints_vel') else torch.rand(N, 38 if 'physics' in k else 6, generator=g) for k in OBSERVATION_KEYS}
+  ts = BatchedTimeStep(torch.randint(0, 3, (N,), dtype=torch.uint8, generator=g), torch.rand(N, generator=g), torch.ones(N), obs)
+  src = dict(step_type=ts.step_type.float().numpy(), reward=ts.reward.numpy(), discount=ts.discount.numpy(),
+             **{k: v.numpy() for k, v in obs.items() if v.numel()})
+  names = bench.dump_outputs(str(tmp_path / 'full'), ts)
+  assert names == sorted(k + '.npy' for k in src)
+  for k, v in src.items():
+    a = np.load(tmp_path / 'full' / f'{k}.npy')
+    assert a.dtype == np.float32 and np.array_equal(a, v), k
+  budget = 100_000
+  for d in ('a', 'b'):
+    names = bench.dump_outputs(str(tmp_path / d), ts, max_bytes=budget)
+    assert names == sorted([k + '.npy' for k in src] + ['env_index.npy'])
+    assert sum(os.path.getsize(tmp_path / d / n) for n in names) <= budget
+  idx = np.load(tmp_path / 'a' / 'env_index.npy')
+  assert idx.dtype == np.float64 and 200 < len(idx) < N and np.all(np.diff(idx) > 0)
+  for k, v in src.items():
+    a = np.load(tmp_path / 'a' / f'{k}.npy')
+    assert np.array_equal(a, v[idx.astype(np.int64)]) and np.array_equal(a, np.load(tmp_path / 'b' / f'{k}.npy')), k
+
+
 def test_bench_gpu_arm_refuses_to_run_without_a_gpu():
   """No CPU fallback: without a CUDA device the GPU arm stops with a message instead of measuring something else."""
   import subprocess, sys
