@@ -396,6 +396,18 @@ struct Handle : HandleBase {
       if (count < (size_t)S.NU * nv) throw std::runtime_error("debug_read: buffer too small");
       if (scene) launch_cast_copy<T, float>(S.warm, dst, (size_t)S.NU * nv, s); else launch_soa_to_rows<T, float>(S.warm, dst, S.N, nv, s);
       launches += 1;
+    } else if (f == "tier") {
+      // solver tier (0, 1, 2) each env was solved in during the last substep (scene_classify_kernel)
+      if (!scene) throw std::runtime_error("debug_read: tier needs a contact scene");
+      if (count < (size_t)S.NU) throw std::runtime_error("debug_read: buffer too small");
+      launch_cast_copy<uint8_t, float>(pipe.tier, dst, S.NU, s);
+      launches += 1;
+    } else if (f == "contacts_width") {
+      // contacts per env the "contacts" probe holds (its rows are 1 + 9 * width floats)
+      if (count < 1) throw std::runtime_error("debug_read: buffer too small");
+      const float w = (float)NCON;
+      CUDA_OK(cudaMemcpyAsync(dst, &w, sizeof w, cudaMemcpyHostToDevice, s));
+      CUDA_OK(cudaStreamSynchronize(s));
     } else if (f == "epahist") {
       if (count < 8) throw std::runtime_error("debug_read: buffer too small");
       int h[8]; float hf[8];
@@ -432,7 +444,7 @@ struct Handle : HandleBase {
       for (int i = 0; i < 16; i++) hf[i] = (float)h[i];
       CUDA_OK(cudaMemcpy(dst, hf, sizeof hf, cudaMemcpyHostToDevice));
     } else if (f == "contacts") {
-      // [N][1 + 9*NCON]: ncon, then (geom1, geom2, dist, pos3, normal3) per contact of the last substep.  The first call only
+      // [N][1 + 9*NCON]: ncon (may exceed NCON), then (geom1, geom2, dist, pos3, normal3) per contact of the last substep.  The first call only
       // enables the probe (the buffer is filled by subsequent steps).
       const size_t need = (size_t)S.NU * (1 + 9 * NCON);
       if (count < need) throw std::runtime_error("debug_read: buffer too small");

@@ -8,7 +8,7 @@
 
 namespace so101 {
 
-constexpr int NCON = 64;         // contacts per env the parity probe (debug_contacts) can report
+constexpr int NCON = 128;        // contacts per env the parity probe (debug_contacts) can report: all CONBUF of them
 constexpr int PAIRCAP = 64;      // candidate geom pairs per env per substep (after the OBB mid phase)
 constexpr int CONBUF = 128;      // raw contacts per env the narrow phase may write between two kernels
 constexpr int EPA_MAXV = 96, EPA_MAXF = 256;

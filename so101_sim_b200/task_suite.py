@@ -383,12 +383,15 @@ class BatchedEnvironment:
 
   def debug_contacts(self):
     """Parity probe: contacts of the last substep, per env a list of (geom1, geom2, dist, pos[3], normal[3]).  The first call
-    enables the probe and returns empty lists."""
-    ncon_max = 64
-    raw = self.debug_read('contacts', 1 + 9 * ncon_max).cpu().numpy()
+    enables the probe and returns empty lists.  Raises if an env had more contacts than the probe holds."""
+    width = int(self.debug_read('contacts_width')[0, 0])
+    raw = self.debug_read('contacts', 1 + 9 * width).cpu().numpy()
     out = []
     for e in range(self.num_envs):
-      n = int(raw[e, 0]); rows = raw[e, 1:1 + 9 * n].reshape(n, 9)
+      n = int(raw[e, 0])
+      if n > width:
+        raise RuntimeError(f'env {e} had {n} contacts, the contact probe holds {width}')
+      rows = raw[e, 1:1 + 9 * n].reshape(n, 9)
       out.append([(int(r[0]), int(r[1]), float(r[2]), r[3:6].copy(), r[6:9].copy()) for r in rows])
     return out
 
