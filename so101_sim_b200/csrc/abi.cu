@@ -81,7 +81,7 @@ static void mm3(const double *a, const double *b, double *r) {
 // Build the description of arm `arm` from the generic blob: joints 6 * arm .. 6 * arm + 5 must be hinges that form a serial chain
 // whose root's parent is static (scene_pbr.xml:74-126), with their dofs / actuators at the same indices.
 template <typename T>
-static void build_arm_model(const Blob &b, ArmModelT<T> &am, int arm = 0) {
+static void build_arm(const Blob &b, ArmModelT<T> &am, int arm = 0) {
   const auto &jt = b.I("jnt_type"), &jb = b.I("jnt_body"), &bp = b.I("body_parent"), &bw = b.I("body_weld");
   const int j0 = NJ * arm;
   if ((int)jt.size() < j0 + NJ) throw std::runtime_error("model has fewer hinge joints than this build's arms need");
@@ -163,12 +163,9 @@ static void build_arm_model(const Blob &b, ArmModelT<T> &am, int arm = 0) {
     const int ga = j0 + a;
     if (b.I("act_jnt")[ga] != ga) throw std::runtime_error("actuator a must drive joint a");
     if (b.F("act_gear")[ga] != 1.0) throw std::runtime_error("actuator gear must be 1");
-    am.gain[a] = (T)b.F("act_gain")[ga]; am.gain_d[a] = b.F("act_gain")[ga];
-    for (int c = 0; c < 3; c++) { am.bias[a][c] = (T)b.F("act_bias")[3 * ga + c]; am.bias_d[a][c] = b.F("act_bias")[3 * ga + c]; }
-    for (int c = 0; c < 2; c++) {
-      am.ctrlrange[a][c] = (T)b.F("act_ctrlrange")[2 * ga + c]; am.forcerange[a][c] = (T)b.F("act_forcerange")[2 * ga + c];
-      am.ctrlrange_d[a][c] = b.F("act_ctrlrange")[2 * ga + c]; am.forcerange_d[a][c] = b.F("act_forcerange")[2 * ga + c];
-    }
+    am.gain_d[a] = b.F("act_gain")[ga];
+    for (int c = 0; c < 3; c++) am.bias_d[a][c] = b.F("act_bias")[3 * ga + c];
+    for (int c = 0; c < 2; c++) { am.ctrlrange_d[a][c] = b.F("act_ctrlrange")[2 * ga + c]; am.forcerange_d[a][c] = b.F("act_forcerange")[2 * ga + c]; }
   }
   am.dt_d = dt;
   for (int c = 0; c < 3; c++) am.gravity[c] = (T)opt[1 + c];
@@ -213,7 +210,7 @@ struct Handle : HandleBase {
     cfg = c;
     nq = b.scalar("nq"); nv = b.scalar("nv"); nu = b.scalar("nu"); nbody = b.scalar("nbody");
     if (nq == NJ && NARM != 1) throw std::runtime_error("the arm-only model needs the one-arm build of the library (libso101_b200.so)");
-    for (int k = 0; k < NARM; k++) { build_arm_model<T>(b, am.arm[k], k); build_arm_model<double>(b, am64.arm[k], k); }
+    for (int k = 0; k < NARM; k++) { build_arm<T>(b, am.arm[k], k); build_arm<double>(b, am64.arm[k], k); }
     if (nq != NJ || c.collide) {
       if (!c.collide) throw std::runtime_error("models with free props need collide=1");
       scene.reset(new SceneModelHost<T>());
@@ -245,10 +242,6 @@ struct Handle : HandleBase {
     S.ring_phys = dalloc<float>((size_t)(c.physics_delay_steps + 1) * (nq + nv) * N);
     S.diverged_count = dalloc<int>(2); S.solver_iter = dalloc<int>(N); S.ncon = dalloc<int>(N); S.dropped_env = dalloc<int>(N);
     sc.nsub = c.n_substeps; sc.last_step = c.last_step; sc.dj = c.joints_delay_steps; sc.dp = c.physics_delay_steps;
-    if (getenv("SO101_PROFILE") && atoi(getenv("SO101_PROFILE"))) S.prof = dalloc<unsigned long long>(16);
-    sc.dbg_env = getenv("SO101_DBG_ENV") ? atoi(getenv("SO101_DBG_ENV")) : -1;
-    sc.dbg_step = getenv("SO101_DBG_STEP") ? atoi(getenv("SO101_DBG_STEP")) : -1;
-    sc.arm_mode = getenv("SO101_ARM_MODE") ? atoi(getenv("SO101_ARM_MODE")) : 4;
     sc.integrator = c.integrator == 1 ? 1 : 0;
     sc.terminate_on_success = c.terminate_on_success; sc.max_iter = c.solver_iterations; sc.tol = c.solver_tolerance;
     for (int i = 0; i < 6; i++) { sc.offsets[i] = c.calibration_offsets[i]; sc.home[i] = c.home_ctrl[i]; }
@@ -408,23 +401,6 @@ struct Handle : HandleBase {
       const float w = (float)NCON;
       CUDA_OK(cudaMemcpyAsync(dst, &w, sizeof w, cudaMemcpyHostToDevice, s));
       CUDA_OK(cudaStreamSynchronize(s));
-    } else if (f == "epahist") {
-      if (count < 8) throw std::runtime_error("debug_read: buffer too small");
-      int h[8]; float hf[8];
-      CUDA_OK(cudaStreamSynchronize(s));
-      scene_epahist<T>(h);
-      for (int i = 0; i < 8; i++) hf[i] = (float)h[i];
-      CUDA_OK(cudaMemcpy(dst, hf, sizeof hf, cudaMemcpyHostToDevice));
-    } else if (f == "nprof") {
-      // narrow-phase warp timing probe (scene_narrow_seq_kernel, SO101_PROFILE=1): 16 counters as floats
-      if (count < 16) throw std::runtime_error("debug_read: buffer too small");
-      unsigned long long h[16]; float hf[16];
-      CUDA_OK(cudaStreamSynchronize(s));
-      scene_nprof<T>(h);
-      h[3] = (h[3] >> 8) * 256 + (h[3] & 0xff);  // (max warp cycles, geom id) stay packed; floats carry them approximately
-      for (int i = 0; i < 16; i++) hf[i] = (float)h[i];
-      hf[6] = (float)(h[3] & 0xff); hf[3] = (float)(h[3] >> 8);
-      CUDA_OK(cudaMemcpy(dst, hf, sizeof hf, cudaMemcpyHostToDevice));
     } else if (f == "dropcat") {
       // 8 drop counters by buffer (see scene_solve.cuh: g_dropcat), since the library was loaded
       if (count < 8) throw std::runtime_error("debug_read: buffer too small");
@@ -432,16 +408,6 @@ struct Handle : HandleBase {
       CUDA_OK(cudaStreamSynchronize(s));
       scene_dropcat<T>(h);
       for (int i = 0; i < 8; i++) hf[i] = (float)h[i];
-      CUDA_OK(cudaMemcpy(dst, hf, sizeof hf, cudaMemcpyHostToDevice));
-    } else if (f == "prof") {
-      // 16 stage-profile accumulators (clock64 sums / counters over all envs since create); needs SO101_PROFILE=1 at create
-      if (!S.prof) throw std::runtime_error("debug_read: create the handle with SO101_PROFILE=1 to enable the stage profile");
-      if (count < 16) throw std::runtime_error("debug_read: buffer too small");
-      unsigned long long h[16];
-      CUDA_OK(cudaStreamSynchronize(s));
-      CUDA_OK(cudaMemcpy(h, S.prof, sizeof h, cudaMemcpyDeviceToHost));
-      float hf[16];
-      for (int i = 0; i < 16; i++) hf[i] = (float)h[i];
       CUDA_OK(cudaMemcpy(dst, hf, sizeof hf, cudaMemcpyHostToDevice));
     } else if (f == "contacts") {
       // [N][1 + 9*NCON]: ncon (may exceed NCON), then (geom1, geom2, dist, pos3, normal3) per contact of the last substep.  The first call only

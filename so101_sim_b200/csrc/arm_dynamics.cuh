@@ -4,7 +4,7 @@
 //   mj_kinematics + mj_comPos  -> arm_fk()
 //   mj_crb (+ armature)        -> arm_crb_rne()   (world-frame composite-rigid-body sweep, tip -> base)
 //   mj_rne (bias forces)       -> arm_crb_rne()   (same sweep; velocity-product accelerations, gravity as base accel)
-//   mj_fwdActuation            -> arm_actuation() (scene_pbr.xml:11: gain 50, bias "0 -50 1", ctrl/force clamps)
+//   mj_fwdActuation            -> arm_actuation_d() (scene_pbr.xml:11: gain 50, bias "0 -50 1", ctrl/force clamps)
 // Templated on the scalar so the same code runs in float32 (north_star dtype) and float64 (tight-parity mode).
 #pragma once
 #include <cuda_runtime.h>
@@ -38,10 +38,8 @@ struct ArmModelT {
   T range[NJ][2];
   int limited[NJ];
   T lim_solimp[NJ][5], lim_K[NJ], lim_B[NJ], invweight0[NJ];
-  // actuators
-  T gain[NJ], bias[NJ][3], ctrlrange[NJ][2], forcerange[NJ][2];
   T gravity[3], dt, solver_scale;  // solver_scale = 1 / (meaninertia * max(1, nv))
-  // float64 copies of what the float64 parts of the float32 path read (actuation and the Euler update, env_state.cuh)
+  // actuators and the Euler update step: float64 in both precisions (env_state.cuh)
   double gain_d[NJ], bias_d[NJ][3], ctrlrange_d[NJ][2], forcerange_d[NJ][2], dt_d;
 };
 
@@ -200,18 +198,8 @@ __device__ __forceinline__ void arm_crb_rne(const ArmModelT<T> &am, const ArmKin
   }
 }
 
-template <typename T>
-__device__ __forceinline__ void arm_actuation(const ArmModelT<T> &am, const T (&q)[NJ], const T (&qd)[NJ], const T (&ctrl)[NJ], T (&frc)[NJ]) {
-#pragma unroll
-  for (int i = 0; i < NJ; i++) {
-    const T c = t_clamp(ctrl[i], am.ctrlrange[i][0], am.ctrlrange[i][1]);
-    const T f = am.gain[i] * c + am.bias[i][0] + am.bias[i][1] * q[i] + am.bias[i][2] * qd[i];
-    frc[i] = t_clamp(f, am.forcerange[i][0], am.forcerange[i][1]);
-  }
-}
-
-// The same actuator model evaluated in float64 on the float64 integration state (the -50 q position feedback would otherwise
-// see the state rounded to float32: 50 * 3e-8 / armature 0.1 = 1.5e-5 rad/s^2 of noise per substep).
+// Actuator forces, evaluated in float64 on the float64 integration state in both precisions (the -50 q position feedback would
+// otherwise see the state rounded to float32: 50 * 3e-8 / armature 0.1 = 1.5e-5 rad/s^2 of noise per substep).
 template <typename T>
 __device__ __forceinline__ void arm_actuation_d(const ArmModelT<T> &am, const double (&q)[NJ], const double (&qd)[NJ], const T (&ctrl)[NJ],
                                                 double (&frc)[NJ]) {

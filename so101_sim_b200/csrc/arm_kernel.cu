@@ -7,8 +7,6 @@
 // per control step (coalesced SoA); nothing else touches HBM.
 #include "arm_kernel.cuh"
 
-#include <type_traits>
-
 namespace so101 {
 
 template <typename T>
@@ -66,12 +64,13 @@ __device__ __forceinline__ void reset_env_arm(const StepCfg &cfg, const EnvState
   write_obs_arm(cfg, S, out, env, 0, q, qd, ctrl, 0.f, 1.f, SO101_STEP_FIRST);
 }
 
-// T = arithmetic of the constraint solver (and of everything else unless stated); TD = arithmetic of the smooth dynamics
-// (FK, CRB, RNE); ACT64 / SOLVE64: actuator model / the M^-1 solve for qacc_smooth in float64; ROUND32: round the state to
-// float32 after every substep (the round-1 behaviour, kept for the error-budget experiment only).  The integration state and
-// the Euler update are float64 in every mode (env_state.cuh).  For T = double all modes are the same code.
-template <typename T, typename TD, bool ACT64, bool SOLVE64, bool ROUND32>
-__global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ ArmModelT<T> am, const __grid_constant__ ArmModelT<TD> amd,
+// T = arithmetic of the friction-loss / limit Newton solve.  The smooth dynamics (FK, CRB, RNE), the actuators, the M^-1 solve
+// for qacc_smooth and the Euler update run in float64 on the float64 state in both precisions (env_state.cuh): measured
+// against the float64 oracle over 100 control steps, 32 envs, float32 throughout drifts to 1.8e-3 relative, float64 smooth
+// dynamics with float32 actuators or M^-1 solve to 1.5e-4 .. 2.3e-4, this split to 9.4e-6, at 481 vs 460 us per 4096-env
+// control step (profiles/r2c_arm_precision.jsonl).  amd: the float64 arm model.
+template <typename T>
+__global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ ArmModelT<T> am, const __grid_constant__ ArmModelT<double> amd,
                                                       const __grid_constant__ StepCfg cfg, const EnvState<T> S, const float *__restrict__ action,
                                                       const so101_step_out out) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
@@ -91,32 +90,21 @@ __global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ A
   int iters = 0;
   bool bad = false;
   for (int sub = 0; sub < cfg.nsub; sub++) {
-    TD qf[NJ], qdf[NJ];
-#pragma unroll
-    for (int i = 0; i < NJ; i++) { qf[i] = (TD)q[i]; qdf[i] = (TD)qd[i]; }
-    ArmKin<TD> k;
-    arm_fk<TD>(amd, qf, k, nullptr);
-    TD Md[21], biasd[NJ];
-    arm_crb_rne(amd, k, qdf, Md, biasd);
+    ArmKin<double> k;
+    arm_fk<double>(amd, q, k, nullptr);
+    double Md[21], biasd[NJ];
+    arm_crb_rne(amd, k, qd, Md, biasd);
     T M[21], qacc_s[NJ];
 #pragma unroll
     for (int i = 0; i < 21; i++) M[i] = (T)Md[i];
-    using TA = typename std::conditional<ACT64, double, T>::type;   // actuator force
-    using TQ = typename std::conditional<SOLVE64, double, T>::type;  // qacc_smooth solve
-    TA frc[NJ];
-    if constexpr (ACT64) arm_actuation_d(am, q, qd, ctrl, frc);
-    else {
-      T qt[NJ], qdt[NJ];
+    double frc[NJ];
+    arm_actuation_d(am, q, qd, ctrl, frc);
+    double L[21], rhs[NJ];
 #pragma unroll
-      for (int i = 0; i < NJ; i++) { qt[i] = (T)q[i]; qdt[i] = (T)qd[i]; }
-      arm_actuation(am, qt, qdt, ctrl, frc);
-    }
-    TQ L[21], rhs[NJ];
-#pragma unroll
-    for (int i = 0; i < 21; i++) L[i] = (TQ)Md[i];
+    for (int i = 0; i < 21; i++) L[i] = Md[i];
     chol6(L);
 #pragma unroll
-    for (int i = 0; i < NJ; i++) rhs[i] = (TQ)((TA)frc[i] - (TA)biasd[i]);
+    for (int i = 0; i < NJ; i++) rhs[i] = frc[i] - biasd[i];
     chol6_solve(L, rhs);
     TS qacc_sd[NJ];
 #pragma unroll
@@ -132,14 +120,11 @@ __global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ A
     iters = arm_solve(am, M, rows, delta, cfg.max_iter, (T)cfg.tol);
     TS corr[NJ] = {TS(0), TS(0), TS(0), TS(0), TS(0), TS(0)};
     if (cfg.integrator == 1) {  // implicitfast: velocity update with (M - h D)^-1 M qacc instead of qacc
-      double fd[NJ];
+      const unsigned vm = arm_actuation_vel_mask(am, frc);
+      double qa[NJ], dv[NJ], cr[NJ];
 #pragma unroll
-      for (int i = 0; i < NJ; i++) fd[i] = (double)frc[i];
-      const unsigned vm = arm_actuation_vel_mask(am, fd);
-      TD qa[NJ], dv[NJ], cr[NJ];
-#pragma unroll
-      for (int i = 0; i < NJ; i++) { qa[i] = (TD)(qacc_sd[i] + (TS)delta[i]); dv[i] = ((vm >> i) & 1u) ? (TD)am.bias_d[i][2] : TD(0); }
-      implicitfast_correction<TD>(Md, dv, (TD)am.dt_d, qa, cr);
+      for (int i = 0; i < NJ; i++) { qa[i] = qacc_sd[i] + (TS)delta[i]; dv[i] = ((vm >> i) & 1u) ? am.bias_d[i][2] : 0.0; }
+      implicitfast_correction<double>(Md, dv, am.dt_d, qa, cr);
 #pragma unroll
       for (int i = 0; i < NJ; i++) corr[i] = (TS)cr[i];
     }
@@ -150,7 +135,6 @@ __global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ A
       bad |= !(t_abs(qacc) < TS(1e10));  // [upstream] mj_checkAcc (also catches NaN)
       qd[i] += am.dt_d * (qacc + corr[i]);  // [upstream] mj_Euler: velocity first, then position with the new velocity
       q[i] += am.dt_d * qd[i];
-      if constexpr (ROUND32) { qd[i] = (TS)(float)qd[i]; q[i] = (TS)(float)q[i]; }
     }
   }
   const int t = S.step[env] + 1;
@@ -184,20 +168,7 @@ void launch_arm_step(const ArmModelT<T> &am, const ArmModelT<double> &am64, cons
   // one env per thread; small batches use 32-thread CTAs so that every one of the 148 SMs gets work
   const int threads = S.N <= 148 * 32 * 4 ? 32 : (S.N <= 148 * 64 * 4 ? 64 : 128);
   const int grid = (S.N + threads - 1) / threads;
-  if constexpr (sizeof(T) == 8) arm_step_kernel<T, T, false, false, false><<<grid, threads, 0, stream>>>(am, am, cfg, S, action, out);
-  else {
-    switch (cfg.arm_mode) {
-      case 0: arm_step_kernel<T, T, false, false, true><<<grid, threads, 0, stream>>>(am, am, cfg, S, action, out); break;
-      case 1: arm_step_kernel<T, T, false, false, false><<<grid, threads, 0, stream>>>(am, am, cfg, S, action, out); break;
-      case 2: arm_step_kernel<T, T, true, false, false><<<grid, threads, 0, stream>>>(am, am, cfg, S, action, out); break;
-      case 3: arm_step_kernel<T, T, true, true, false><<<grid, threads, 0, stream>>>(am, am, cfg, S, action, out); break;
-      // product default (mode 4): smooth dynamics, actuators, M^-1 solve and Euler update in float64; the friction-loss / limit
-      // Newton solve in float32.  Measured against the float64 oracle over 100 control steps, 32 envs (tools/exp_arm_precision.py,
-      // profiles/r2a_arm_precision.jsonl): mode 0 (all float32) 1.8e-3, modes 1-3 1.5e-4 .. 2.3e-4, mode 4 9.4e-6 relative,
-      // at 481 vs 460 us per 4096-env control step.
-      default: arm_step_kernel<T, double, true, true, false><<<grid, threads, 0, stream>>>(am, am64, cfg, S, action, out); break;
-    }
-  }
+  arm_step_kernel<T><<<grid, threads, 0, stream>>>(am, am64, cfg, S, action, out);
 }
 template <typename T>
 void launch_arm_reset(const StepCfg &cfg, const EnvState<T> &S, const uint8_t *mask, const so101_step_out &out, cudaStream_t stream) {

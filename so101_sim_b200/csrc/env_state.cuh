@@ -11,7 +11,7 @@ namespace so101 {
 // (FK, CRB, RNE, actuators, M^-1), and the semi-implicit Euler update in float64: the reference's actuators are anti-damped
 // (bias +1 * qvel, scene_pbr.xml:11) and amplify a perturbation ~300x over 100 control steps, so that neither a float32 state
 // (1.8e-3 relative error after 100 steps) nor float32 smooth dynamics on a float64 state (1.6e-4) meet north_star's 1e-4;
-// float64 smooth dynamics + float32 solver give 9e-6 (tools/exp_arm_precision.py; DESIGN.md section 2).
+// float64 smooth dynamics + float32 solver give 9e-6 (profiles/r2c_arm_precision.jsonl; DESIGN.md section 2).
 using TS = double;
 
 // On-device episode initialisation of the hand-over tasks (so100_hand_over.py:208-229,320-323; [upstream] dm_control
@@ -63,16 +63,13 @@ struct EnvState {
   int *solver_iter;                 // [N] Newton iterations of the last substep (parity/diagnostics)
   int *ncon;                        // [N] contacts of the last substep
   int *dropped_env;                 // [N] contacts / candidate pairs this env lost to a full buffer since create (see so101_counters)
-  unsigned long long *prof;         // optional [16] stage-profile accumulators (SO101_PROFILE=1), see scene_kernel.inl
   float *dbg_contacts;              // optional [N][1 + 9*NCON] parity probe (null unless requested)
 };
 
 struct StepCfg {
   int nsub, last_step, dj, dp, terminate_on_success, max_iter;
   int integrator;  // 0 = semi-implicit Euler (the reference's default, scene_pbr.xml sets none), 1 = implicitfast (north_star)
-  int arm_mode;  // developer switch (SO101_ARM_MODE): which parts of the float32 arm path run in float64, see arm_kernel.cu
   float tol;
-  int dbg_env, dbg_step;  // developer probe: device printf of one env's manifold inputs (SO101_DBG_ENV / SO101_DBG_STEP)
   float offsets[6], home[6];
 };
 

@@ -211,7 +211,7 @@ __device__ __forceinline__ void msupport_seq(const SceneModel<T> &sm, Shape<T> &
 
 // boolean GJK; mirrors gjk_intersect() of the oracle.  Uniform control flow across the warp.
 template <typename T>
-__device__ __forceinline__ int gjk_intersect(const SceneModel<T> &sm, Shape<T> &A, Shape<T> &B, MPoint<T> *S, int &np, int &iters) {
+__device__ __forceinline__ int gjk_intersect(const SceneModel<T> &sm, Shape<T> &A, Shape<T> &B, MPoint<T> *S, int &np) {
   T d[3];
   sub3(d, B.center, A.center);
   if (dot3(d, d) < T(1e-20)) { d[0] = T(1); d[1] = T(0); d[2] = T(0); }
@@ -219,7 +219,6 @@ __device__ __forceinline__ int gjk_intersect(const SceneModel<T> &sm, Shape<T> &
   #pragma unroll 1
   for (int it = 0; it < 64; it++) {
     MPoint<T> p;
-    iters = it + 1;
     msupport_seq(sm, A, B, d, p);
     if (dot3(p.w, d) < T(0)) { np = n; return 0; }
     S[n++] = p;

@@ -205,22 +205,17 @@ __device__ __forceinline__ int epa_end(CollideScratch<T> &cs, const EpaState<T> 
 
 template <typename T>
 __device__ __noinline__ int epa_seq(const SceneModel<T> &sm, CollideScratch<T> &cs, Shape<T> &A, Shape<T> &B, const MPoint<T> *S, int n, T *normal,
-                                    T &depth, T *pa, T *pb, int &iters) {
+                                    T &depth, T *pa, T *pb) {
   EpaState<T> st;
-  iters = 0;
   if (!epa_begin(sm, cs, A, B, S, n, st)) return 0;
   int r;
 #pragma unroll 1
   do { r = epa_step(sm, cs, A, B, st); } while (r == 0);
-  iters = st.it;
   if (r < 0) return 0;
   return epa_end(cs, st, normal, depth, pa, pb);
 }
 
 // vertices of s within delta of the support plane along dir -> CCW 2-D convex polygon in (t1,t2) with heights
-#ifndef EPA_ITCAP
-#define EPA_ITCAP 80
-#endif
 constexpr int SCANW = 8;  // hull vertices examined per trip of the slab scan
 template <typename T>
 __device__ __noinline__ int feature_seq(const SceneModel<T> &sm, CollideScratch<T> &cs, Shape<T> &s, const T *dir, const T *t1, const T *t2, T delta,
@@ -492,10 +487,9 @@ __device__ __forceinline__ void finish_convex_pair(const SceneModel<T> &sm, Coll
 
 template <typename T>
 __device__ __noinline__ void collide_convex_seq(const SceneModel<T> &sm, CollideScratch<T> &cs, Shape<T> &A, Shape<T> &B, const MPoint<T> *S, int n,
-                                                PairContacts<T> &pc, int &eit, long long &t_epa) {
+                                                PairContacts<T> &pc) {
   T normal[3], depth, pa[3], pb[3];
-  const int ok = epa_seq(sm, cs, A, B, S, n, normal, depth, pa, pb, eit);
-  t_epa = clock64();  // (stage probe: when this lane left EPA)
+  const int ok = epa_seq(sm, cs, A, B, S, n, normal, depth, pa, pb);
   finish_convex_pair(sm, cs, A, B, ok, normal, depth, pa, pb, pc);
 }
 

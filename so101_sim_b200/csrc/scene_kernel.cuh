@@ -136,8 +136,4 @@ template <typename T>
 void launch_debug_overlap(const double *cases, int n, uint8_t *out, cudaStream_t stream);
 template <typename T>
 void scene_dropcat(int out[8]);
-template <typename T>
-void scene_epahist(int out[8]);
-template <typename T>
-void scene_nprof(unsigned long long out[16]);
 }  // namespace so101

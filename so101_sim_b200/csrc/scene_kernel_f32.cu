@@ -8,6 +8,4 @@ template void launch_settle_enter<float>(const EnvState<float> &, unsigned, cuda
 template void launch_settle_leave<float>(const EnvState<float> &, cudaStream_t);
 template void launch_debug_overlap<float>(const double *, int, uint8_t *, cudaStream_t);
 template void scene_dropcat<float>(int *);
-template void scene_epahist<float>(int *);
-template void scene_nprof<float>(unsigned long long *);
 }  // namespace so101

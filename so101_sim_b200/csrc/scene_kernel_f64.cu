@@ -8,6 +8,4 @@ template void launch_settle_enter<double>(const EnvState<double> &, unsigned, cu
 template void launch_settle_leave<double>(const EnvState<double> &, cudaStream_t);
 template void launch_debug_overlap<double>(const double *, int, uint8_t *, cudaStream_t);
 template void scene_dropcat<double>(int *);
-template void scene_epahist<double>(int *);
-template void scene_nprof<double>(unsigned long long *);
 }  // namespace so101

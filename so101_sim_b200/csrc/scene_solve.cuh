@@ -19,8 +19,6 @@ namespace so101 {
 // where contacts / candidate pairs were dropped by a full buffer since the library was loaded (diagnostics):
 // 0 NOUT per pair, 1 CANDCAP, 2 PAIRCAP, 3 work-queue capacity, 4 CONBUF raw contacts, 5 Jacobian block pool
 __device__ int g_dropcat[8];
-__device__ unsigned long long g_nprof[16];  // narrow-phase warp timing probe (SO101_PROFILE=1): see scene_narrow_seq_kernel
-__device__ int g_epahist[8];  // EPA iterations per call: <=2, <=5, <=10, <=20, <=40, < cap, cap, (unused)
 #define DROPCAT(i, n) atomicAdd(&g_dropcat[i], (int)(n))
 
 constexpr int NH = NV * (NV + 1) / 2;  // 171 packed lower-triangular entries
@@ -336,7 +334,6 @@ __device__ __noinline__ void rows_line(S &s, const ArmLane<T> &al, T impratio, T
     }
   }
   c += warp_sum(lc); g += warp_sum(lg); h += warp_sum(lh);
-  if (s.profon && lane == 0) s.prof[13] += 1;  // P_LINE
 }
 
 template <typename T>

@@ -434,14 +434,12 @@ def test_checkpoint_carries_the_placement_machinery(built):
 @pytest.mark.parametrize('precision', ['f32', 'f64'])
 def test_two_launch_narrow_phase_is_bit_identical(built, monkeypatch, precision):
   """Groups of 32768+ envs run the narrow phase as two launches (scene_epa_kernel: EPA as a per-lane state machine with pairs
-  taken from a cursor; scene_narrow_split_kernel<1>: manifold / plane contacts) instead of the fused thread-per-pair kernel.
-  Forced on at 64 envs (SO101_NARROW_SPLIT = smallest group size that uses it), with both EPA variants, the states after 25
-  random-action control steps must equal the fused kernel's bit for bit, and the launch counter must show the extra launch."""
+  taken from a cursor; scene_manifold_kernel: manifold / plane contacts) instead of the fused thread-per-pair kernel.
+  Forced on at 64 envs (SO101_NARROW_SPLIT = smallest group size that uses it), the states after 25 random-action control
+  steps must equal the fused kernel's bit for bit, and the launch counter must show the extra launch."""
   results = []
-  for split, refill in (('1000000000', None), ('1', '20'), ('1', '3'), ('1', '0')):
+  for split in ('1000000000', '1'):
     monkeypatch.setenv('SO101_NARROW_SPLIT', split)
-    if refill is None: monkeypatch.delenv('SO101_EPA_REFILL', raising=False)
-    else: monkeypatch.setenv('SO101_EPA_REFILL', refill)
     env = _env(built, num_envs=64, precision=precision)
     _initial(env, seed=11)
     acts = _actions(env, 25, seed=5)
