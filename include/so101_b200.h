@@ -165,6 +165,40 @@ int so101_kernel_times(so101_handle h, int enable, double ms_out[11], uint64_t l
  * caller-owned device buffer of `count` floats.  Used by the parity tests only. */
 int so101_debug_read(so101_handle h, const char *field, float *dst_dev, size_t count, void *stream);
 
+/* End-effector queries.  The tool centre point (TCP) is a point fixed in each arm's Fixed_Jaw body (the body of its fifth hinge,
+ * Wrist_Roll) at tcp_offset (metres, Fixed_Jaw frame); its orientation is the Fixed_Jaw frame.  Both functions run FK of the
+ * arms in float64 in both precisions, one thread per (env, arm), only for the user envs.  They are enqueued on the caller's
+ * stream, never synchronise the host, write only the caller's buffers and leave the handle's state and its captured step
+ * graphs untouched.  narm = 1, or 2 for the two-arm build. */
+typedef struct so101_ee_params {
+  float tcp_offset[3];  /* TCP in the Fixed_Jaw frame (the library's Python layer derives the default from the jaw pads) */
+  int iterations;       /* Levenberg-Marquardt iterations (>= 0; default 16) */
+  float damping;        /* lambda (metres, > 0): the step solves (J J^T + lambda^2 I) y = e */
+  float w_rot;          /* metres per radian of orientation error (>= 0; ignored without a target orientation) */
+  float max_step;       /* per-joint clamp of one iteration's step (rad, > 0) */
+  float tolerance;      /* stop early once |e| (metres, orientation part weighted by w_rot) < tolerance; 0 = never */
+} so101_ee_params;
+/* TCP pose of every user env and arm: the current joint state (from_ctrl = 0) or the current commanded joint targets
+ * (from_ctrl != 0: ctrl, i.e. the last action plus the calibration offsets).  pos_dev [N,narm,3] float32 world position,
+ * quat_dev [N,narm,4] float32 world orientation, wxyz (MuJoCo convention) with w >= 0 (nullable).  The reference has no
+ * counterpart: reading the gripper pose there means restating the arm's kinematics on physics.named.data.xpos / xmat. */
+int so101_ee_pose(so101_handle h, int from_ctrl, const float tcp_offset[3], float *pos_dev, float *quat_dev, void *stream);
+/* Batched inverse kinematics to joint-target actions.  Replaces the reference planner's geometric stand-in
+ * inverse_kinematics_approximate (examples/automated_lerobot_dataset_generator.py:188-212), which does not place the jaws at
+ * the target.  Damped least squares on the five arm hinges of each arm (the jaw is excluded), started from the env's current
+ * joint state or from seed_q_dev ([N,nu] float32 joint positions, nullable):
+ *   e = (p_target - p_tcp, w_rot * rotation vector of R_target R_tcp^T), Jacobian columns (a_i x (p_tcp - p_i), w_rot * a_i),
+ *   dq = J^T y with (J J^T + damping^2 I) y = e, each component clamped to +-max_step, then q clamped to the joint range,
+ * for p->iterations iterations (fewer once |e| < tolerance).  target_pos_dev [N,narm,3]; target_quat_dev [N,narm,4] wxyz,
+ * nullable = position only (w_rot is then 0).  action_out_dev [N,nu] float32 receives ACTIONS, q - calibration_offsets, since
+ * the step adds the offsets back; its jaw entries are gripper_dev [N,narm] unchanged (nullable: the current commanded jaw
+ * target minus its offset).  err_out_dev [N,narm,2] (nullable): final position error (m) and orientation error (rad, 0 without
+ * a target orientation).  Targets are not validated: an unreachable target gives finite joint targets inside the joint range
+ * and shows only in err_out_dev.  The parameters are validated (negative return on a bad one).  Deterministic: the same
+ * inputs give the same bits. */
+int so101_ee_ik(so101_handle h, const float *target_pos_dev, const float *target_quat_dev, const float *gripper_dev, const float *seed_q_dev,
+                const so101_ee_params *p, float *action_out_dev, float *err_out_dev, void *stream);
+
 /* Parity probe without a handle: the device's 6-axis box overlap test (the reward geometry, so101_sim/utils/oobb_utils.py:202-273)
  * on n box pairs, rows of 20 doubles (pos 3, quat 4 wxyz, half 3 of box A, then of box B), evaluated in float32 or float64
  * (precision = 32 / 64) -> out[i] in {0, 1}.  Used by the golden-vector test of the reward geometry only. */

@@ -4,6 +4,7 @@
 #include <nvtx3/nvToolsExt.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -14,6 +15,7 @@
 #include "../../include/so101_b200.h"
 #include "arm_kernel.cuh"
 #include "blob.hpp"
+#include "ee_kernel.cuh"
 #include "layout_kernels.cuh"
 #include "scene_kernel.cuh"
 
@@ -62,6 +64,8 @@ struct HandleBase {
   virtual uint64_t diverged() = 0;
   virtual size_t checkpoint_bytes() = 0;
   virtual void checkpoint(void *buf_dev, size_t bytes, bool load, cudaStream_t s) = 0;
+  virtual void ee_pose(bool from_ctrl, const float tcp[3], float *pos, float *quat, cudaStream_t s) = 0;
+  virtual void ee_ik(const EeIkArgs &a, cudaStream_t s) = 0;
   KernelTimer timer;
   std::vector<TierExec> tiers;  // one per pipeline group
 };
@@ -543,6 +547,20 @@ struct Handle : HandleBase {
     for (const Seg &g : segs) { CUDA_OK(cudaMemcpyAsync(g.p, buf + off, g.bytes, cudaMemcpyDeviceToDevice, s)); off += pad16(g.bytes); }
     settle_epoch = hd.settle_epoch; steps = hd.steps;
   }
+  // ---- end-effector queries: read the state / commanded targets, write the caller's buffers only (no graph, no handle state)
+  EeSrc ee_src() const {
+    EeSrc e{S.qpos, S.ctrl, sizeof(T) == sizeof(double), scene ? 1 : 0, S.N, S.NU, nq, {}};
+    for (int i = 0; i < NJ; i++) e.offsets[i] = sc.offsets[i];
+    return e;
+  }
+  void ee_pose(bool from_ctrl, const float tcp[3], float *pos, float *quat, cudaStream_t s) override {
+    launch_ee_pose(am64, ee_src(), from_ctrl ? 1 : 0, tcp, pos, quat, s);
+    launches += 1;
+  }
+  void ee_ik(const EeIkArgs &a, cudaStream_t s) override {
+    launch_ee_ik(am64, ee_src(), a, s);
+    launches += 1;
+  }
   uint64_t diverged() override {
     int v[2] = {0, 0};
     cudaMemcpy(v, S.diverged_count, 2 * sizeof(int), cudaMemcpyDeviceToHost);
@@ -752,6 +770,30 @@ int so101_debug_overlap(int precision, int device, const double *cases_dev, int 
   if (precision == 32) launch_debug_overlap<float>(cases_dev, n, out_dev, (cudaStream_t)stream);
   else launch_debug_overlap<double>(cases_dev, n, out_dev, (cudaStream_t)stream);
   return cudaPeekAtLastError() == cudaSuccess ? 0 : -3;
+}
+int so101_ee_pose(so101_handle h, int from_ctrl, const float tcp_offset[3], float *pos_dev, float *quat_dev, void *stream) {
+  API_BEGIN(h)
+  NvtxRange range_("so101_ee_pose");
+  if (!tcp_offset || !pos_dev) throw std::runtime_error("null pointer");
+  H->ee_pose(from_ctrl != 0, tcp_offset, pos_dev, quat_dev, (cudaStream_t)stream);
+  API_END()
+}
+int so101_ee_ik(so101_handle h, const float *target_pos_dev, const float *target_quat_dev, const float *gripper_dev, const float *seed_q_dev,
+                const so101_ee_params *p, float *action_out_dev, float *err_out_dev, void *stream) {
+  API_BEGIN(h)
+  NvtxRange range_("so101_ee_ik");
+  if (!target_pos_dev || !p || !action_out_dev) throw std::runtime_error("null pointer");
+  if (p->iterations < 0) throw std::runtime_error("iterations must be >= 0");
+  if (!(std::isfinite(p->damping) && p->damping > 0)) throw std::runtime_error("damping must be finite and > 0");
+  if (!(std::isfinite(p->w_rot) && p->w_rot >= 0)) throw std::runtime_error("w_rot must be finite and >= 0");
+  if (!(std::isfinite(p->max_step) && p->max_step > 0)) throw std::runtime_error("max_step must be finite and > 0");
+  if (!(p->tolerance >= 0)) throw std::runtime_error("tolerance must be >= 0");
+  for (int c = 0; c < 3; c++)
+    if (!std::isfinite(p->tcp_offset[c])) throw std::runtime_error("tcp_offset must be finite");
+  EeIkArgs a{target_pos_dev, target_quat_dev, gripper_dev, seed_q_dev, {p->tcp_offset[0], p->tcp_offset[1], p->tcp_offset[2]}, p->iterations,
+             (double)p->damping, (double)p->w_rot, (double)p->max_step, (double)p->tolerance, action_out_dev, err_out_dev};
+  H->ee_ik(a, (cudaStream_t)stream);
+  API_END()
 }
 int so101_debug_read(so101_handle h, const char *field, float *dst_dev, size_t count, void *stream) {
   API_BEGIN(h)

@@ -27,15 +27,15 @@ TABLE_Z = 0.42  # automated_lerobot_dataset_generator.py:68,76,197
 
 
 def convert_to_lerobot_format(joints_pos: torch.Tensor, action: Optional[torch.Tensor], frame_index: int, episode_index: int,
-                              device=None) -> Dict[str, Any]:
-  """so101_lerobot_wrapper.py:77-122 for a batch: `joints_pos` [N,6] (the delayed observation), `action` [N,6] or None (the
-  reset observation echoes a zero action)."""
+                              device=None, action_dim: int = 6) -> Dict[str, Any]:
+  """so101_lerobot_wrapper.py:77-122 for a batch: `joints_pos` [N,6] (the delayed observation), `action` [N,action_dim] or None
+  (the reset observation echoes a zero action)."""
   n = joints_pos.shape[0]
   dev = joints_pos.device if device is None else torch.device(device)
   out: Dict[str, Any] = {}
   # copies: the env re-uses its observation buffers from step to step, a recorded frame must not alias them
   out['observation.state'] = joints_pos.to(device=dev, dtype=torch.float32, copy=True)
-  out['action'] = torch.zeros(n, 6, device=dev) if action is None else action.to(device=dev, dtype=torch.float32, copy=True)
+  out['action'] = torch.zeros(n, action_dim, device=dev) if action is None else action.to(device=dev, dtype=torch.float32, copy=True)
   out['timestamp'] = torch.full((n,), frame_index * 0.1, dtype=torch.float32, device=dev)  # (sic: 0.1, not the 0.02 s control step)
   out['frame_index'] = torch.full((n,), frame_index, dtype=torch.long, device=dev)
   out['episode_index'] = torch.full((n,), episode_index, dtype=torch.long, device=dev)
@@ -46,12 +46,27 @@ def convert_to_lerobot_format(joints_pos: torch.Tensor, action: Optional[torch.T
 
 
 class BatchedSO101LeRobotWrapper:
-  """N lockstep copies of SO101LeRobotWrapper (scripts/so101_lerobot_wrapper.py:15-188)."""
+  """N lockstep copies of SO101LeRobotWrapper (scripts/so101_lerobot_wrapper.py:15-188).
+
+  action_space='joint' (default): actions are joint targets [N,6], as in the reference.  action_space='ee_delta': actions are
+  end-effector deltas [N,4] per arm, (dx, dy, dz) of the tool centre point in metres and the jaw action, run through
+  BatchedEnvironment.step_ee from the current TCP (`ee_base`), clipped to the `ee_workspace` box ((lo[3], hi[3]) or None), with
+  the IK parameters `ee_params`; the recorded 'action' is the [N,4] delta action."""
+
+  ACTION_SPACES = ('joint', 'ee_delta')
+  action_space = 'joint'
 
   def __init__(self, task_name: str = 'SO100HandOverBanana', num_envs: int = 1, cameras: tuple = (), camera_resolution: tuple = (480, 640),
-               time_limit: float = 30.0, device: str = 'cuda:0', seed: int | None = None, reset_rounds: int = 1, **env_kwargs):
+               time_limit: float = 30.0, device: str = 'cuda:0', seed: int | None = None, reset_rounds: int = 1, action_space: str = 'joint',
+               ee_workspace=None, ee_base: str = 'state', ee_params: Optional[dict] = None, **env_kwargs):
     if cameras:
       raise NotImplementedError('camera rendering is out of scope of the B200 path: pass cameras=()')
+    if action_space not in self.ACTION_SPACES:
+      raise ValueError(f'action_space must be one of {self.ACTION_SPACES}, got {action_space!r}')
+    if ee_base not in ('state', 'command'):
+      raise ValueError("ee_base must be 'state' or 'command'")
+    self.action_space = action_space
+    self.ee_workspace, self.ee_base, self.ee_params = ee_workspace, ee_base, dict(ee_params or {})
     self.device = device
     self.cameras = tuple(cameras)
     self.camera_resolution = camera_resolution
@@ -70,9 +85,12 @@ class BatchedSO101LeRobotWrapper:
     ts = self.env.reset()
     self.frame_index = 0
     self.start_time = 0.0
-    return convert_to_lerobot_format(ts.observation['joints_pos'], None, self.frame_index, self.episode_index, self.device)
+    return convert_to_lerobot_format(ts.observation['joints_pos'], None, self.frame_index, self.episode_index, self.device,
+                                     4 * self.env.narm if self.action_space == 'ee_delta' else 6)
 
   def step(self, action) -> Dict[str, Any]:
+    if self.action_space == 'ee_delta':
+      return self._step_ee(action)
     action = torch.as_tensor(np.asarray(action) if not isinstance(action, torch.Tensor) else action, dtype=torch.float32)
     if action.dim() == 1:
       action = action.expand(self.num_envs, 6)
@@ -80,6 +98,19 @@ class BatchedSO101LeRobotWrapper:
     self.last_timestep = ts
     self.frame_index += 1
     return convert_to_lerobot_format(ts.observation['joints_pos'], action, self.frame_index, self.episode_index, self.device)
+
+  def _step_ee(self, action) -> Dict[str, Any]:
+    na = self.env.narm
+    action = (action if isinstance(action, torch.Tensor) else torch.as_tensor(np.asarray(action))).to(device=self.device, dtype=torch.float32)
+    if action.dim() == 1:
+      action = action.expand(self.num_envs, 4 * na)
+    if tuple(action.shape) != (self.num_envs, 4 * na):
+      raise ValueError(f'ee_delta actions must have shape [{self.num_envs}, {4 * na}] or [{4 * na}], got {list(action.shape)}')
+    a = action.reshape(self.num_envs, na, 4)
+    ts = self.env.step_ee(a[..., :3], a[..., 3], base=self.ee_base, workspace=self.ee_workspace, **self.ee_params)
+    self.last_timestep = ts
+    self.frame_index += 1
+    return convert_to_lerobot_format(ts.observation['joints_pos'], action, self.frame_index, self.episode_index, self.device, 4 * na)
 
   def collect_episode(self, actions, save_path: Optional[str] = None) -> List[Dict[str, Any]]:
     """so101_lerobot_wrapper.py:124-158; `actions` is a sequence of [N,6] (or [6]) actions."""
@@ -92,6 +123,10 @@ class BatchedSO101LeRobotWrapper:
     return episode
 
   def get_action_spec(self) -> Dict[str, Any]:  # so101_lerobot_wrapper.py:160-168
+    if self.action_space == 'ee_delta':
+      lo, hi = (None, None) if self.ee_workspace is None else (np.asarray(self.ee_workspace[0]), np.asarray(self.ee_workspace[1]))
+      return {'shape': (4 * self.env.narm,), 'dtype': np.float32, 'workspace_low': lo, 'workspace_high': hi,
+              'names': [f'{n}{"" if self.env.narm == 1 else f"_{k}"}' for k in range(self.env.narm) for n in ('delta_x', 'delta_y', 'delta_z', 'gripper')]}
     return {'shape': (6,), 'dtype': np.float32, 'low': -1.0, 'high': 1.0,
             'names': ['rotation', 'pitch', 'elbow', 'wrist_pitch', 'wrist_roll', 'jaw']}
 

@@ -30,3 +30,31 @@ def read_blob(path: str) -> dict[str, np.ndarray]:
     name, dt, cnt, off = struct.unpack_from('<24sIIQ', raw, 16 + 40 * i)
     out[name.rstrip(b'\0').decode()] = np.frombuffer(raw, dtype=np.float64 if dt == 0 else np.int32, count=cnt, offset=off).copy()
   return out
+
+
+def tcp_offset(model: dict[str, np.ndarray], arm: int = 0) -> np.ndarray:
+  """Default tool centre point of arm `arm`, in the frame of its Fixed_Jaw body (the body of the arm's fifth hinge, Wrist_Roll):
+  the midpoint of the centroid of the Fixed_Jaw's box pads and the centroid of the Moving_Jaw's box pads at jaw angle 0 (carried
+  into the Fixed_Jaw frame through the Moving_Jaw's body_pos / body_quat and the jaw hinge at qpos0 -> 0).  Metres, float64 [3]."""
+  box = 4   # geom type code of a box in the blob (tools/compile_model.py GEOM_BOX)
+  jb = model['jnt_body']
+  if len(jb) < 6 * arm + 6:
+    raise ValueError(f'model has no arm {arm}')
+  fixed, moving, jaw = int(jb[6 * arm + 4]), int(jb[6 * arm + 5]), 6 * arm + 5
+  gb, gt, gp = model['geom_body'], model['geom_type'], model['geom_pos'].reshape(-1, 3)
+  pads_f, pads_m = gp[(gb == fixed) & (gt == box)], gp[(gb == moving) & (gt == box)]
+  if not len(pads_f) or not len(pads_m):
+    raise ValueError(f'arm {arm}: the jaws have no box pads to define the tool centre point')
+  if int(model['body_parent'][moving]) != fixed:
+    raise ValueError(f'arm {arm}: the Moving_Jaw is not a child of the Fixed_Jaw')
+  w, x, y, z = model['body_quat'].reshape(-1, 4)[moving] / np.linalg.norm(model['body_quat'].reshape(-1, 4)[moving])
+  R = np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+  # jaw angle 0: rotate the Moving_Jaw frame about its hinge (anchored at the body origin) by 0 - qpos0
+  ax = model['jnt_axis'].reshape(-1, 3)[jaw]
+  th = -float(model['qpos0'][jaw])
+  K = np.array([[0, -ax[2], ax[1]], [ax[2], 0, -ax[0]], [-ax[1], ax[0], 0]])
+  Rj = np.eye(3) + np.sin(th) * K + (1 - np.cos(th)) * K @ K
+  moving_in_fixed = model['body_pos'].reshape(-1, 3)[moving] + R @ Rj @ pads_m.mean(axis=0)
+  return 0.5 * (pads_f.mean(axis=0) + moving_in_fixed)
