@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define SO101_ABI_VERSION 4
+#define SO101_ABI_VERSION 5
 
 /* dm_env.StepType values (reference TimeStep.step_type) */
 #define SO101_STEP_FIRST 0
@@ -161,7 +161,7 @@ int so101_counters(so101_handle h, uint64_t out[6]);
  * recorded events.  No reference counterpart: measurement support for bench.py's roofline leg. */
 int so101_kernel_times(so101_handle h, int enable, double ms_out[11], uint64_t launches_out[11]);
 
-/* Debug/parity probe: copy one internal structure-of-arrays field ("qacc", "ncon", "solver_iter", ...) of all envs to a
+/* Debug/parity probe: copy one internal per-env field ("warm", "ncon", "solver_iter", ...) of all envs, row-major, to a
  * caller-owned device buffer of `count` floats.  Used by the parity tests only. */
 int so101_debug_read(so101_handle h, const char *field, float *dst_dev, size_t count, void *stream);
 

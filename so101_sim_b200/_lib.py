@@ -80,7 +80,7 @@ def load(narm: int = 1) -> ctypes.CDLL:
   L.so101_debug_read.restype = ci; L.so101_debug_read.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t, vp]
   L.so101_ee_pose.restype = ci; L.so101_ee_pose.argtypes = [vp, ci, ctypes.POINTER(ctypes.c_float * 3), vp, vp, vp]
   L.so101_ee_ik.restype = ci; L.so101_ee_ik.argtypes = [vp, vp, vp, vp, vp, ctypes.POINTER(EEParams), vp, vp, vp]
-  if L.so101_abi_version() != 4:
+  if L.so101_abi_version() != 5:
     raise RuntimeError(f'{path}: ABI version mismatch')
   _libs[narm] = L
   return L

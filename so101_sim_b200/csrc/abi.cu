@@ -1,5 +1,5 @@
 // C-ABI implementation (include/so101_b200.h): handle life cycle, model upload, kernel launches.
-// PyTorch owns every tensor that crosses this boundary; the handle owns only its SoA state and scratch.
+// PyTorch owns every tensor that crosses this boundary; the handle owns only its state (env_state.cuh) and scratch.
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 
@@ -182,7 +182,7 @@ template <typename T>
 struct Handle : HandleBase {
   ArmSetT<T> am;
   ArmSetT<double> am64;  // float64 arm models for the float64 parts of the float32 path
-  std::unique_ptr<SceneModelHost<T>> scene;  // non-null: full contact scene (warp per env, row-major state)
+  std::unique_ptr<SceneModelHost<T>> scene;  // non-null: full contact scene (warp per env)
   EnvState<T> S{};
   PipeBuf<T> pipe{};                 // per-env scratch shared by all groups
   std::vector<PipeBuf<T>> groups;    // per-group queues / counters (views of `pipe` with their own work lists)
@@ -251,7 +251,7 @@ struct Handle : HandleBase {
     for (int i = 0; i < 6; i++) { sc.offsets[i] = c.calibration_offsets[i]; sc.home[i] = c.home_ctrl[i]; }
     // default initial state: qpos0, zero velocity
     std::vector<TS> q0(nq * N);
-    for (int k = 0; k < nq; k++) for (size_t e = 0; e < N; e++) q0[scene ? e * nq + k : k * N + e] = (TS)b.F("qpos0")[k];
+    for (size_t e = 0; e < N; e++) for (int k = 0; k < nq; k++) q0[e * nq + k] = (TS)b.F("qpos0")[k];
     CUDA_OK(cudaMemcpy(S.init_qpos, q0.data(), q0.size() * sizeof(TS), cudaMemcpyHostToDevice));
     d_action = dalloc<float>(NA * N);
     use_graph = !(getenv("SO101_GRAPH") && atoi(getenv("SO101_GRAPH")) == 0);
@@ -301,7 +301,7 @@ struct Handle : HandleBase {
   template <typename A>
   void set_state_any(const A *q, const A *v, bool initial, cudaStream_t s) {
     auto put = [&](const A *rows, TS *dst, int k) {
-      if (scene) launch_cast_copy<A, TS>(rows, dst, (size_t)S.NU * k, s); else launch_rows_to_soa<A, TS>(rows, dst, S.N, k, s);
+      launch_cast_copy<A, TS>(rows, dst, (size_t)S.NU * k, s);
       launches += 1;
     };
     put(q, S.qpos, nq); put(v, S.qvel, nv);
@@ -329,21 +329,18 @@ struct Handle : HandleBase {
     for (int r = 0; r < rounds; r++) {
       const float *qr = q + (size_t)r * NU * nq, *vr = v + (size_t)r * NU * nv;
       TS *dq = S.init_qpos + (size_t)r * N * nq, *dv = S.init_qvel + (size_t)r * N * nv;
-      if (scene) { launch_cast_copy<float, TS>(qr, dq, NU * nq, s); launch_cast_copy<float, TS>(vr, dv, NU * nv, s); }
-      else { launch_rows_to_soa<float, TS>(qr, dq, S.N, nq, s); launch_rows_to_soa<float, TS>(vr, dv, S.N, nv, s); }
+      launch_cast_copy<float, TS>(qr, dq, NU * nq, s); launch_cast_copy<float, TS>(vr, dv, NU * nv, s);
       launches += 2;
     }
     S.npool = rounds;
     CUDA_OK(cudaMemsetAsync(S.episode, 0, sizeof(int) * N, s));
   }
   void get_state(float *q, float *v, cudaStream_t s) override {
-    if (scene) { launch_cast_copy<TS, float>(S.qpos, q, (size_t)S.NU * nq, s); launch_cast_copy<TS, float>(S.qvel, v, (size_t)S.NU * nv, s); }
-    else { launch_soa_to_rows<TS, float>(S.qpos, q, S.N, nq, s); launch_soa_to_rows<TS, float>(S.qvel, v, S.N, nv, s); }
+    launch_cast_copy<TS, float>(S.qpos, q, (size_t)S.NU * nq, s); launch_cast_copy<TS, float>(S.qvel, v, (size_t)S.NU * nv, s);
     launches += 2;
   }
   void get_state_f64(double *q, double *v, cudaStream_t s) override {
-    if (scene) { launch_cast_copy<TS, double>(S.qpos, q, (size_t)S.NU * nq, s); launch_cast_copy<TS, double>(S.qvel, v, (size_t)S.NU * nv, s); }
-    else { launch_soa_to_rows<TS, double>(S.qpos, q, S.N, nq, s); launch_soa_to_rows<TS, double>(S.qvel, v, S.N, nv, s); }
+    launch_cast_copy<TS, double>(S.qpos, q, (size_t)S.NU * nq, s); launch_cast_copy<TS, double>(S.qvel, v, (size_t)S.NU * nv, s);
     launches += 2;
   }
   void reset(const uint8_t *mask, const so101_step_out &out, cudaStream_t s) override {
@@ -391,7 +388,7 @@ struct Handle : HandleBase {
       launches += 1;
     } else if (f == "warm") {
       if (count < (size_t)S.NU * nv) throw std::runtime_error("debug_read: buffer too small");
-      if (scene) launch_cast_copy<T, float>(S.warm, dst, (size_t)S.NU * nv, s); else launch_soa_to_rows<T, float>(S.warm, dst, S.N, nv, s);
+      launch_cast_copy<T, float>(S.warm, dst, (size_t)S.NU * nv, s);
       launches += 1;
     } else if (f == "tier") {
       // solver tier (0, 1, 2) each env was solved in during the last substep (scene_classify_kernel)
@@ -549,7 +546,7 @@ struct Handle : HandleBase {
   }
   // ---- end-effector queries: read the state / commanded targets, write the caller's buffers only (no graph, no handle state)
   EeSrc ee_src() const {
-    EeSrc e{S.qpos, S.ctrl, sizeof(T) == sizeof(double), scene ? 1 : 0, S.N, S.NU, nq, {}};
+    EeSrc e{S.qpos, S.ctrl, sizeof(T) == sizeof(double), S.NU, nq, {}};
     for (int i = 0; i < NJ; i++) e.offsets[i] = sc.offsets[i];
     return e;
   }

@@ -4,64 +4,33 @@
 // M^-1, friction-loss/limit Newton solve, semi-implicit Euler} ([upstream] mj_step; Euler is MuJoCo's default
 // integrator, scene_pbr.xml:4), observation delay rings (so100_task.py:189-210), reward (= 0 for the base task,
 // so100_task.py:289-290), time limit and dm_control's auto-reset — is ONE launch.  State is read once and written once
-// per control step (coalesced SoA); nothing else touches HBM.
+// per control step (its row of every state array); nothing else touches HBM.
 #include "arm_kernel.cuh"
 
 namespace so101 {
 
+// What write_obs reads: the env's state and commanded targets, held in registers by the kernels below.
 template <typename T>
-__device__ __forceinline__ void write_obs_arm(const StepCfg &cfg, const EnvState<T> &S, const so101_step_out &out, int env, int t,
-                                              const TS (&q)[NJ], const TS (&qd)[NJ], const T (&ctrl)[NJ], float reward, float discount,
-                                              uint8_t step_type) {
-  const int N = S.N;
-  // delay rings: slot t % (D+1) holds the value after control step t; read max(t-D, 0)  (INITIAL_VALUE padding,
-  // task_suite.py:154)
-  const int dj = cfg.dj + 1, dp = cfg.dp + 1;
-  float *rj = S.ring_joints + (size_t)(t % dj) * 6 * N;
-  float *rp = S.ring_phys + (size_t)(t % dp) * 12 * N;
-#pragma unroll
-  for (int i = 0; i < NJ; i++) {
-    rj[i * N + env] = (float)q[i];
-    rp[i * N + env] = (float)q[i];
-    rp[(6 + i) * N + env] = (float)qd[i];
-  }
-  const int tj = t - cfg.dj > 0 ? t - cfg.dj : 0, tp = t - cfg.dp > 0 ? t - cfg.dp : 0;
-  const float *dj_src = S.ring_joints + (size_t)(tj % dj) * 6 * N;
-  const float *dp_src = S.ring_phys + (size_t)(tp % dp) * 12 * N;
-#pragma unroll
-  for (int i = 0; i < NJ; i++) {
-    if (out.commanded_joints_pos) out.commanded_joints_pos[env * 6 + i] = (float)ctrl[i];
-    if (out.undelayed_joints_pos) out.undelayed_joints_pos[env * 6 + i] = (float)q[i];
-    if (out.joints_pos) out.joints_pos[env * 6 + i] = tj == t ? (float)q[i] : dj_src[i * N + env];
-    if (out.physics_state) { out.physics_state[env * 12 + i] = (float)q[i]; out.physics_state[env * 12 + 6 + i] = (float)qd[i]; }
-  }
-  if (out.delayed_physics_state) {
-#pragma unroll
-    for (int i = 0; i < 12; i++) out.delayed_physics_state[env * 12 + i] = tp == t ? (i < 6 ? (float)q[i] : (float)qd[i - 6]) : dp_src[i * N + env];
-  }
-  if (out.reward) out.reward[env] = reward;
-  if (out.discount) out.discount[env] = discount;
-  if (out.step_type) out.step_type[env] = step_type;
-}
+struct ArmObs { const TS *q, *qd; const T *ctrl; };
 
 template <typename T>
 __device__ __forceinline__ void reset_env_arm(const StepCfg &cfg, const EnvState<T> &S, const so101_step_out &out, int env) {
-  const int N = S.N;
   TS q[NJ], qd[NJ];
   T ctrl[NJ];
   const int ep = S.episode[env];
-  const size_t pool = (size_t)(ep % S.npool) * NJ * N;  // reset pool entry of this episode
+  const size_t pool = ((size_t)(ep % S.npool) * S.N + env) * NJ;  // reset pool entry of this episode
+  const int row = env * NJ;
   S.episode[env] = ep + 1;
 #pragma unroll
   for (int i = 0; i < NJ; i++) {
-    q[i] = S.init_qpos[pool + i * N + env]; qd[i] = S.init_qvel[pool + i * N + env];
+    q[i] = S.init_qpos[pool + i]; qd[i] = S.init_qvel[pool + i];
     ctrl[i] = (T)cfg.home[i] + (T)cfg.offsets[i];  // so100_task.py:316-317
-    S.qpos[i * N + env] = q[i]; S.qvel[i * N + env] = qd[i]; S.warm[i * N + env] = T(0); S.ctrl[i * N + env] = ctrl[i];
+    S.qpos[row + i] = q[i]; S.qvel[row + i] = qd[i]; S.warm[row + i] = T(0); S.ctrl[row + i] = ctrl[i];
   }
   S.step[env] = 0;
   S.needs_reset[env] = 0;
   // FIRST TimeStep: reward / discount are None in dm_env; the batched tensors carry 0 / 1.
-  write_obs_arm(cfg, S, out, env, 0, q, qd, ctrl, 0.f, 1.f, SO101_STEP_FIRST);
+  write_obs<NJ, NJ, NJ, 1>(cfg, S, out, ArmObs<T>{q, qd, ctrl}, env, 0, 0.f, 1.f, SO101_STEP_FIRST, 0);
 }
 
 // T = arithmetic of the friction-loss / limit Newton solve.  The smooth dynamics (FK, CRB, RNE), the actuators, the M^-1 solve
@@ -74,17 +43,17 @@ __global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ A
                                                       const __grid_constant__ StepCfg cfg, const EnvState<T> S, const float *__restrict__ action,
                                                       const so101_step_out out) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
-  const int N = S.N;
-  if (env >= N) return;
+  if (env >= S.N) return;
   if (S.needs_reset[env]) {  // dm_control: the step() after a LAST step resets and returns FIRST
     reset_env_arm(cfg, S, out, env);
     return;
   }
+  const int row = env * NJ;   // (32-bit: at 255 registers a 64-bit index costs the float32 kernel stack and spills)
   TS q[NJ], qd[NJ];
   T warm[NJ], ctrl[NJ];
 #pragma unroll
   for (int i = 0; i < NJ; i++) {
-    q[i] = S.qpos[i * N + env]; qd[i] = S.qvel[i * N + env]; warm[i] = S.warm[i * N + env];
+    q[i] = S.qpos[row + i]; qd[i] = S.qvel[row + i]; warm[i] = S.warm[row + i];
     ctrl[i] = (T)action[env * 6 + i] + (T)cfg.offsets[i];  // before_step: action + homing offsets, unclamped
   }
   int iters = 0;
@@ -149,9 +118,9 @@ __global__ void __launch_bounds__(128) arm_step_kernel(const __grid_constant__ A
   S.needs_reset[env] = st == SO101_STEP_LAST;
 #pragma unroll
   for (int i = 0; i < NJ; i++) {
-    S.qpos[i * N + env] = q[i]; S.qvel[i * N + env] = qd[i]; S.warm[i * N + env] = warm[i]; S.ctrl[i * N + env] = ctrl[i];
+    S.qpos[row + i] = q[i]; S.qvel[row + i] = qd[i]; S.warm[row + i] = warm[i]; S.ctrl[row + i] = ctrl[i];
   }
-  write_obs_arm(cfg, S, out, env, t, q, qd, ctrl, reward, discount, st);
+  write_obs<NJ, NJ, NJ, 1>(cfg, S, out, ArmObs<T>{q, qd, ctrl}, env, t, reward, discount, st, 0);
 }
 
 template <typename T>

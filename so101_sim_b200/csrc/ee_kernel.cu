@@ -15,10 +15,10 @@ constexpr int IK_JOINTS = NJ - 1;  // the five arm hinges; the jaw is left to th
 
 __device__ __forceinline__ double load_joint(const EeSrc &s, int env, int j, bool from_ctrl) {
   if (from_ctrl) {
-    const size_t i = s.rows ? (size_t)env * NA + j : (size_t)j * s.N + env;
+    const size_t i = (size_t)env * NA + j;
     return s.ctrl_f64 ? static_cast<const double *>(s.ctrl)[i] : (double)static_cast<const float *>(s.ctrl)[i];
   }
-  return s.qpos[s.rows ? (size_t)env * s.nq + j : (size_t)j * s.N + env];
+  return s.qpos[(size_t)env * s.nq + j];
 }
 
 // Unit quaternion (w, x, y, z), w >= 0, of a row-major rotation matrix (Shepperd's method: divide by the largest of the four

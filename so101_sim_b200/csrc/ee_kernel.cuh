@@ -4,14 +4,13 @@
 
 namespace so101 {
 
-// Where the arm joint angles of the user envs live: the float64 state (arm-only handles: SoA [k][N]; contact scenes: rows
-// [N][nq]) and the commanded targets S.ctrl (same layouts with NA columns, float32 or float64 as the handle's precision).
+// Where the arm joint angles of the user envs live: the float64 state S.qpos [N][nq] and the commanded targets S.ctrl [N][NA]
+// (float32 or float64 as the handle's precision).
 struct EeSrc {
   const double *qpos;
   const void *ctrl;
   int ctrl_f64;   // S.ctrl holds doubles (precision 64) rather than floats
-  int rows;       // 1 = row layout [N][nq] / [N][NA] (contact scene), 0 = SoA [k][N] (arm-only)
-  int N, NU, nq;  // N = all envs (the SoA stride), NU = user envs
+  int NU, nq;     // NU = user envs
   float offsets[NJ];  // calibration offsets: ctrl = action + offsets
 };
 

@@ -1,5 +1,6 @@
-// Device-resident state of N lockstep environments, structure-of-arrays: field[k][env] so that a warp touching the
-// same component of 32 consecutive envs issues one coalesced 128 B (f32) / 256 B (f64) request.
+// Device-resident state of N lockstep environments.  Every per-env array is stored in rows, field[env][k], for the arm-only
+// model and the contact scene alike; the delay rings are [D+1][env][k] and the reset pool [npool][env][k].  Checkpoints are
+// byte copies of these arrays.
 #pragma once
 #include <cstdint>
 #include "../../include/so101_b200.h"
@@ -49,16 +50,16 @@ struct EnvState {
                                     //   initial states or reset pool are installed)
   int *ring_ctr;                    // [RC_N]
   PlacementCfg place;
-  TS *qpos, *qvel;                  // [nq][N], [nv][N]
-  T *warm;                          // [nv][N]  (qacc_warmstart)
-  TS *init_qpos, *init_qvel;        // reset pool [npool][...same layout as qpos / qvel...]: episode e of an env starts from entry e % npool
+  TS *qpos, *qvel;                  // [N][nq], [N][nv]
+  T *warm;                          // [N][nv]  (qacc_warmstart)
+  TS *init_qpos, *init_qvel;        // reset pool [npool][N][nq], [npool][N][nv]: episode e of an env starts from entry e % npool
   int npool;                        // entries in the reset pool (>= 1)
   int *episode;                     // [N] resets this env has gone through (selects the pool entry)
-  T *ctrl;                          // [6][N]
+  T *ctrl;                          // [N][nu]
   int *step;                        // [N] control steps since reset
   uint8_t *needs_reset;             // [N] previous step was LAST (dm_control auto-reset on next step)
-  float *ring_joints;               // [Dj+1][6][N]
-  float *ring_phys;                 // [Dp+1][nq+nv][N]
+  float *ring_joints;               // [Dj+1][N][nu]
+  float *ring_phys;                 // [Dp+1][N][nq+nv]
   int *diverged_count;              // [1]
   int *solver_iter;                 // [N] Newton iterations of the last substep (parity/diagnostics)
   int *ncon;                        // [N] contacts of the last substep
@@ -72,5 +73,42 @@ struct StepCfg {
   float tol;
   float offsets[6], home[6];
 };
+
+// The observations of one env's TimeStep after control step t (t = 0: the FIRST TimeStep of an episode), its reward, discount
+// and step type, and step t's entry of the two delay rings.  Ring slot t % (D+1) holds the value after control step t; a
+// delayed block reads slot max(t - D, 0), so the first D steps of an episode see the initial value (INITIAL_VALUE padding,
+// task_suite.py:154).  LANES threads share one env and `lane` is this thread's index among them: 32 in the scene kernels (a
+// warp per env), 1 in the arm-only kernel (a thread per env).  s.q, s.qd and s.ctrl are the env's state and commanded targets
+// as the caller's kernel holds them; every value written is their float32 rounding.
+template <int NQ_, int NV_, int NU_, int LANES, typename T, typename SC>
+__device__ void write_obs(const StepCfg &cfg, const EnvState<T> &S, const so101_step_out &out, const SC &s, int env, int t, float reward,
+                          float discount, uint8_t st, int lane) {
+  constexpr int SD = NQ_ + NV_;
+  const int dj = cfg.dj + 1, dp = cfg.dp + 1;
+  const size_t N = S.N;
+  float *rj = S.ring_joints + ((size_t)(t % dj) * N + env) * NU_;
+  float *rp = S.ring_phys + ((size_t)(t % dp) * N + env) * SD;
+  const int tj = t - cfg.dj > 0 ? t - cfg.dj : 0, tp = t - cfg.dp > 0 ? t - cfg.dp : 0;
+  const float *sj = S.ring_joints + ((size_t)(tj % dj) * N + env) * NU_;
+  const float *sp = S.ring_phys + ((size_t)(tp % dp) * N + env) * SD;
+  for (int i = lane; i < SD; i += LANES) {
+    const float v = i < NQ_ ? (float)s.q[i] : (float)s.qd[i - NQ_];
+    rp[i] = v;
+    if (out.physics_state) out.physics_state[(size_t)env * SD + i] = v;
+    if (out.delayed_physics_state) out.delayed_physics_state[(size_t)env * SD + i] = tp == t ? v : sp[i];
+  }
+  for (int i = lane; i < NU_; i += LANES) {
+    const float v = (float)s.q[i];
+    rj[i] = v;
+    if (out.undelayed_joints_pos) out.undelayed_joints_pos[(size_t)env * NU_ + i] = v;
+    if (out.joints_pos) out.joints_pos[(size_t)env * NU_ + i] = tj == t ? v : sj[i];
+    if (out.commanded_joints_pos) out.commanded_joints_pos[(size_t)env * NU_ + i] = (float)s.ctrl[i];
+  }
+  if (lane == 0) {
+    if (out.reward) out.reward[env] = reward;
+    if (out.discount) out.discount[env] = discount;
+    if (out.step_type) out.step_type[env] = st;
+  }
+}
 
 }  // namespace so101

@@ -1,23 +1,9 @@
-// Boundary layout conversion: row-major [N,k] tensors (PyTorch side) <-> structure-of-arrays [k][N] (handle side).
+// Element-wise copies with a type conversion between the caller's row-major [N,k] tensors and the handle's state.
 #pragma once
 #include <cuda_runtime.h>
 
 namespace so101 {
 
-template <typename A, typename T>
-__global__ void rows_to_soa_kernel(const A *__restrict__ rows, T *__restrict__ soa, int N, int k) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;  // index into the SoA array: coalesced stores
-  if (i >= N * k) return;
-  const int c = i / N, e = i % N;
-  soa[i] = (T)rows[(size_t)e * k + c];
-}
-template <typename T, typename U>
-__global__ void soa_to_rows_kernel(const T *__restrict__ soa, U *__restrict__ rows, int N, int k) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;  // index into the SoA array: coalesced loads
-  if (i >= N * k) return;
-  const int c = i / N, e = i % N;
-  rows[(size_t)e * k + c] = (U)soa[i];
-}
 __global__ void int_to_float_kernel(const int *__restrict__ src, float *__restrict__ dst, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) dst[i] = (float)src[i];
@@ -30,16 +16,6 @@ __global__ void cast_copy_kernel(const A *__restrict__ src, B *__restrict__ dst,
 template <typename A, typename B>
 inline void launch_cast_copy(const A *src, B *dst, size_t n, cudaStream_t s) {
   cast_copy_kernel<A, B><<<(unsigned)((n + 255) / 256), 256, 0, s>>>(src, dst, n);
-}
-template <typename A, typename T>
-inline void launch_rows_to_soa(const A *rows, T *soa, int N, int k, cudaStream_t s) {
-  const int n = N * k;
-  rows_to_soa_kernel<A, T><<<(n + 255) / 256, 256, 0, s>>>(rows, soa, N, k);
-}
-template <typename T, typename U>
-inline void launch_soa_to_rows(const T *soa, U *rows, int N, int k, cudaStream_t s) {
-  const int n = N * k;
-  soa_to_rows_kernel<T, U><<<(n + 255) / 256, 256, 0, s>>>(soa, rows, N, k);
 }
 inline void launch_int_to_float(const int *src, float *dst, int n, cudaStream_t s) {
   int_to_float_kernel<<<(n + 255) / 256, 256, 0, s>>>(src, dst, n);

@@ -10,8 +10,8 @@
 #include "scene_model.cuh"
 
 namespace so101 {
-// Scene-kernel state layout is array-of-rows ([N][nq] etc.): one warp owns one env and reads its row with one
-// coalesced request (the arm-only kernel, one THREAD per env, uses [k][N] instead).
+// The scene kernels keep the env state in rows (env_state.cuh): one warp owns one env and reads its row with one coalesced
+// request.
 
 // Per-env record written by the thread-per-env kinematics + smooth-dynamics kernel and read by the solve kernels:
 // joint anchors 18, joint axes 18, arm mass matrix 21, prop mass blocks 2 x 21, qacc_smooth 18, arm rows 24

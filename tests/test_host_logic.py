@@ -18,16 +18,19 @@ def test_time_limit_step_matches_reference_accumulation():
 
 
 def test_library_exports_every_declared_symbol(built):
-  """Every function declared in include/so101_b200.h must be exported by the in-tree .so (no compute calls here)."""
+  """Every function declared in include/so101_b200.h must be exported by the in-tree .so, which reports the header's ABI
+  version (no compute calls here)."""
   from so101_sim_b200 import _lib
   hdr = open(os.path.join(ROOT, 'include', 'so101_b200.h')).read()
   declared = set(re.findall(r'\b(so101_[a-z0-9_]+)\s*\(', hdr))
+  abi = int(re.search(r'#define SO101_ABI_VERSION (\d+)', hdr).group(1))
+  assert abi == 5
   assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
   for path in (_lib.LIB_PATH, _lib.LIB_PATH_2ARM):   # one-arm build and the two-arm build of the same sources
     L = ctypes.CDLL(path)
     for sym in declared:
       assert hasattr(L, sym), (path, sym)
-    assert L.so101_abi_version() == 4
+    assert L.so101_abi_version() == abi
 
 
 def test_create_fails_loudly_without_gpu(built):
