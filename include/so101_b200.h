@@ -29,6 +29,9 @@ extern "C" {
 #define SO101_STEP_MID 1
 #define SO101_STEP_LAST 2
 
+/* contact force sensors a handle holds at most (so101_contact_sensors) */
+#define SO101_MAX_CONTACT_SENSORS 16
+
 typedef struct so101_env *so101_handle;
 
 /* Per-step outputs: device pointers into caller-owned row-major tensors, N = num_envs.  Any pointer may be NULL
@@ -164,6 +167,31 @@ int so101_kernel_times(so101_handle h, int enable, double ms_out[11], uint64_t l
 /* Debug/parity probe: copy one internal per-env field ("warm", "ncon", "solver_iter", ...) of all envs, row-major, to a
  * caller-owned device buffer of `count` floats.  Used by the parity tests only. */
 int so101_debug_read(so101_handle h, const char *field, float *dst_dev, size_t count, void *stream);
+
+/* Contact force sensors (MuJoCo's mj_contactForce summed over a body pair, with its `touch` / `contact` sensor values).  A sensor
+ * is an ordered pair of disjoint, non-empty body sets (A, B), given as two 32-bit masks of body ids (bit b = body b of the
+ * model), A first.  After every so101_step each sensor gives each user env one float32 row of 5 values, read from the contacts
+ * of the LAST substep of the step - exactly those the Newton solve used (contacts dropped by a full buffer, or whose Jacobian
+ * blocks did not fit the solver's pool, are not included; friction-loss and limit rows are not contacts):
+ *   [0..2] net force on A from B, world frame, newtons;  [3] sum of the normal forces (>= 0);  [4] number of contacts.
+ * Sign: for a contact between geom1 (body b1) and geom2 (body b2) with cone force f in the contact frame (normal from geom1 to
+ * geom2, tangent 1, tangent 2), the force on b2 from b1 is F = f0 n + f1 t1 + f2 t2; the contact adds +F if b2 is in A and b1 in
+ * B, -F if b1 is in A and b2 in B.  Torsional and rolling components are torques and are not reported.  f is the cone force at
+ * the solver's final iterate.  Rows read all zeros for envs that return FIRST from the step (auto-reset), envs reset by
+ * so101_reset or so101_sample_and_settle, envs whose step ended by divergence, and every env after so101_checkpoint_load until
+ * the next step (the sensor configuration is not part of a checkpoint).  Arithmetic runs in the handle's precision, in a fixed
+ * order: the same inputs give the same bits.
+ * so101_contact_sensors sets n <= SO101_MAX_CONTACT_SENSORS sensors, masks_host[k] = {mask A, mask B}; n = 0 turns them off
+ * (the default: the step then does no sensor work).  Returns negative for a handle without a contact scene, n out of range, an
+ * empty mask, overlapping masks or a body >= nbody.  It drops the handle's captured step graphs.  The first call with n > 0
+ * allocates the readout buffer (cudaMalloc, zero-filled, like the other lazily allocated buffers of a handle); later calls do no
+ * device work and never synchronise.  The readout has the new layout from the next step on: read before it, it holds the
+ * previous configuration's rows (zeros before any step).  With sensors on, a step adds one memset of the readout to its graph
+ * (no kernel launch).
+ * so101_contact_sensors_read copies the [N][n][5] float32 readout of the last step to dst_dev (count floats, at least N * n * 5)
+ * with cudaMemcpyAsync on the caller's stream. */
+int so101_contact_sensors(so101_handle h, int n, const uint32_t masks_host[][2]);
+int so101_contact_sensors_read(so101_handle h, float *dst_dev, size_t count, void *stream);
 
 /* End-effector queries.  The tool centre point (TCP) is a point fixed in each arm's Fixed_Jaw body (the body of its fifth hinge,
  * Wrist_Roll) at tcp_offset (metres, Fixed_Jaw frame); its orientation is the Fixed_Jaw frame.  Both functions run FK of the

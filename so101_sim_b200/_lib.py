@@ -38,7 +38,9 @@ class EEParams(ctypes.Structure):
 EXPORTS = ('so101_abi_version', 'so101_create', 'so101_destroy', 'so101_last_error', 'so101_dims', 'so101_set_initial_state',
            'so101_reset', 'so101_step', 'so101_get_state', 'so101_set_state', 'so101_get_state_f64', 'so101_step_host',
            'so101_counters', 'so101_debug_read', 'so101_kernel_times', 'so101_set_reset_pool', 'so101_set_state_f64', 'so101_debug_overlap', 'so101_sample_and_settle', 'so101_placement_stats', 'so101_get_episode_steps', 'so101_set_episode_steps',
-           'so101_checkpoint_size', 'so101_checkpoint_save', 'so101_checkpoint_load', 'so101_ee_pose', 'so101_ee_ik')
+           'so101_checkpoint_size', 'so101_checkpoint_save', 'so101_checkpoint_load', 'so101_ee_pose', 'so101_ee_ik',
+           'so101_contact_sensors', 'so101_contact_sensors_read')
+MAX_CONTACT_SENSORS = 16   # SO101_MAX_CONTACT_SENSORS
 
 _libs = {}
 
@@ -80,6 +82,8 @@ def load(narm: int = 1) -> ctypes.CDLL:
   L.so101_debug_read.restype = ci; L.so101_debug_read.argtypes = [vp, ctypes.c_char_p, vp, ctypes.c_size_t, vp]
   L.so101_ee_pose.restype = ci; L.so101_ee_pose.argtypes = [vp, ci, ctypes.POINTER(ctypes.c_float * 3), vp, vp, vp]
   L.so101_ee_ik.restype = ci; L.so101_ee_ik.argtypes = [vp, vp, vp, vp, vp, ctypes.POINTER(EEParams), vp, vp, vp]
+  L.so101_contact_sensors.restype = ci; L.so101_contact_sensors.argtypes = [vp, ci, vp]
+  L.so101_contact_sensors_read.restype = ci; L.so101_contact_sensors_read.argtypes = [vp, vp, ctypes.c_size_t, vp]
   if L.so101_abi_version() != 5:
     raise RuntimeError(f'{path}: ABI version mismatch')
   _libs[narm] = L

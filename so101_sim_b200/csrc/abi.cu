@@ -66,6 +66,8 @@ struct HandleBase {
   virtual void checkpoint(void *buf_dev, size_t bytes, bool load, cudaStream_t s) = 0;
   virtual void ee_pose(bool from_ctrl, const float tcp[3], float *pos, float *quat, cudaStream_t s) = 0;
   virtual void ee_ik(const EeIkArgs &a, cudaStream_t s) = 0;
+  virtual void contact_sensors(int n, const uint32_t (*masks)[2]) = 0;
+  virtual void contact_sensors_read(float *dst, size_t count, cudaStream_t s) = 0;
   KernelTimer timer;
   std::vector<TierExec> tiers;  // one per pipeline group
 };
@@ -346,6 +348,7 @@ struct Handle : HandleBase {
   void reset(const uint8_t *mask, const so101_step_out &out, cudaStream_t s) override {
     if (scene) launch_scene_reset<T>(sc, S, mask, out, s); else launch_arm_reset<T>(sc, S, mask, out, s);
     launches += 1;
+    if (sc.nsensor) { launch_zero_rows(S.sensors, mask, S.NU, 5 * sc.nsensor, s); launches += 1; }   // reset envs read zero sensors
   }
   void step(const float *action, const so101_step_out &out, cudaStream_t s) override {
     if (!scene) { timer.begin(4, s); launch_arm_step<T>(am.arm[0], am64.arm[0], sc, S, action, out, s); timer.end(4, s); launches += 1; steps += 1; return; }
@@ -543,6 +546,32 @@ struct Handle : HandleBase {
     size_t off = pad16(sizeof hd);
     for (const Seg &g : segs) { CUDA_OK(cudaMemcpyAsync(g.p, buf + off, g.bytes, cudaMemcpyDeviceToDevice, s)); off += pad16(g.bytes); }
     settle_epoch = hd.settle_epoch; steps = hd.steps;
+    // the contact sensor readout is not part of a checkpoint: zero until the next step
+    if (sc.nsensor) CUDA_OK(cudaMemsetAsync(S.sensors, 0, sizeof(float) * 5 * (size_t)S.NU * sc.nsensor, s));
+  }
+  // ---- contact force sensors (scene_kernel.inl: contact_sensor_pass)
+  void contact_sensors(int n, const uint32_t (*m)[2]) override {
+    if (!scene) throw std::runtime_error("contact sensors need a model with a contact scene");
+    if (n < 0 || n > SO101_MAX_CONTACT_SENSORS) throw std::runtime_error("contact sensors: n must be in 0 .. " + std::to_string(SO101_MAX_CONTACT_SENSORS));
+    if (n > 0 && !m) throw std::runtime_error("contact sensors: null masks");
+    const uint32_t bodies = nbody >= 32 ? ~0u : (1u << nbody) - 1u;
+    for (int k = 0; k < n; k++) {
+      const uint32_t a = m[k][0], b = m[k][1];
+      if (!a || !b) throw std::runtime_error("contact sensor " + std::to_string(k) + ": empty body set");
+      if (a & b) throw std::runtime_error("contact sensor " + std::to_string(k) + ": the two body sets overlap");
+      if ((a | b) & ~bodies) throw std::runtime_error("contact sensor " + std::to_string(k) + ": body id >= nbody");
+    }
+    // the readout buffer holds the largest configuration, so reconfiguring never reallocates (every step zeroes its rows first)
+    if (n > 0 && !S.sensors) S.sensors = dalloc<float>((size_t)S.NU * SO101_MAX_CONTACT_SENSORS * 5);
+    sc.nsensor = n;
+    for (int k = 0; k < SO101_MAX_CONTACT_SENSORS; k++) { sc.sensor_mask[k][0] = k < n ? m[k][0] : 0u; sc.sensor_mask[k][1] = k < n ? m[k][1] : 0u; }
+    invalidate_graphs();
+  }
+  void contact_sensors_read(float *dst, size_t count, cudaStream_t s) override {
+    if (!scene) throw std::runtime_error("contact sensors need a model with a contact scene");
+    const size_t need = (size_t)S.NU * sc.nsensor * 5;
+    if (count < need) throw std::runtime_error("contact sensors: buffer too small (N * n * 5 floats)");
+    if (need) CUDA_OK(cudaMemcpyAsync(dst, S.sensors, need * sizeof(float), cudaMemcpyDeviceToDevice, s));
   }
   // ---- end-effector queries: read the state / commanded targets, write the caller's buffers only (no graph, no handle state)
   EeSrc ee_src() const {
@@ -790,6 +819,17 @@ int so101_ee_ik(so101_handle h, const float *target_pos_dev, const float *target
   EeIkArgs a{target_pos_dev, target_quat_dev, gripper_dev, seed_q_dev, {p->tcp_offset[0], p->tcp_offset[1], p->tcp_offset[2]}, p->iterations,
              (double)p->damping, (double)p->w_rot, (double)p->max_step, (double)p->tolerance, action_out_dev, err_out_dev};
   H->ee_ik(a, (cudaStream_t)stream);
+  API_END()
+}
+int so101_contact_sensors(so101_handle h, int n, const uint32_t masks_host[][2]) {
+  API_BEGIN(h)
+  H->contact_sensors(n, masks_host);
+  API_END()
+}
+int so101_contact_sensors_read(so101_handle h, float *dst_dev, size_t count, void *stream) {
+  API_BEGIN(h)
+  if (!dst_dev) throw std::runtime_error("null pointer");
+  H->contact_sensors_read(dst_dev, count, (cudaStream_t)stream);
   API_END()
 }
 int so101_debug_read(so101_handle h, const char *field, float *dst_dev, size_t count, void *stream) {

@@ -65,6 +65,7 @@ struct EnvState {
   int *ncon;                        // [N] contacts of the last substep
   int *dropped_env;                 // [N] contacts / candidate pairs this env lost to a full buffer since create (see so101_counters)
   float *dbg_contacts;              // optional [N][1 + 9*NCON] parity probe (null unless requested)
+  float *sensors;                   // contact sensor readout [NU][StepCfg::nsensor][5] (null until sensors are first configured)
 };
 
 struct StepCfg {
@@ -72,6 +73,9 @@ struct StepCfg {
   int integrator;  // 0 = semi-implicit Euler (the reference's default, scene_pbr.xml sets none), 1 = implicitfast (north_star)
   float tol;
   float offsets[6], home[6];
+  // contact force sensors (so101_contact_sensors): body masks A, B of each sensor; nsensor = 0 turns the sensor pass off
+  int nsensor;
+  unsigned sensor_mask[SO101_MAX_CONTACT_SENSORS][2];
 };
 
 // The observations of one env's TimeStep after control step t (t = 0: the FIRST TimeStep of an episode), its reward, discount

@@ -47,6 +47,9 @@ struct SolveScratch {
   union V {
     struct Con { T pos[3][NC], frame[9][NC], dist[NC]; int g1[NC], g2[NC]; } con;  // gathered contacts (until the rows are built)
     struct Ls { T jv[6][NC], frc[6][NC]; } ls;                                     // J search, cone forces (Newton iterations)
+    // contact sensor pass after the solve (scene_kernel.inl): per solver index the world force on body[1] from body[0] and the
+    // normal force, the two bodies (-1: contact not in the solve), and the raw slot the contact came from
+    struct Sens { T f[4][NC]; int body[2][NC], slot[NC]; } sens;
   } v;
 };
 

@@ -58,3 +58,29 @@ def tcp_offset(model: dict[str, np.ndarray], arm: int = 0) -> np.ndarray:
   Rj = np.eye(3) + np.sin(th) * K + (1 - np.cos(th)) * K @ K
   moving_in_fixed = model['body_pos'].reshape(-1, 3)[moving] + R @ Rj @ pads_m.mean(axis=0)
   return 0.5 * (pads_f.mean(axis=0) + moving_in_fixed)
+
+
+BODY_SET_NAMES = ('fixed_jaw', 'moving_jaw', 'gripper', 'arm', 'object', 'container', 'static')
+
+
+def body_set(model: dict[str, np.ndarray], name: str, arm: int = 0) -> list[int]:
+  """Body ids of a named part of the model, read from the blob's own tables: 'fixed_jaw' / 'moving_jaw' (the bodies of arm
+  `arm`'s fifth and sixth hinges), 'gripper' (both jaws), 'arm' (the bodies of the arm's six hinges), 'object' / 'container'
+  (the two props), 'static' (every body without a joint: the world, the arm bases, the table and the fixed furniture)."""
+  jb, nbody = model['jnt_body'], int(model['nbody'][0])
+  if name in ('fixed_jaw', 'moving_jaw', 'gripper', 'arm'):
+    narm = int(model['nu'][0]) // 6
+    if not 0 <= arm < narm:
+      raise ValueError(f'model has no arm {arm} (it has {narm})')
+    j0 = 6 * arm
+    ids = {'fixed_jaw': [j0 + 4], 'moving_jaw': [j0 + 5], 'gripper': [j0 + 4, j0 + 5], 'arm': list(range(j0, j0 + 6))}[name]
+    return [int(jb[j]) for j in ids]
+  if name in ('object', 'container'):
+    pb = model['prop_body']
+    p = 0 if name == 'object' else 1
+    if len(pb) <= p:
+      raise ValueError(f'model has no {name} prop')
+    return [int(pb[p])]
+  if name == 'static':
+    return [b for b in range(nbody) if int(model['body_jntnum'][b]) == 0]
+  raise ValueError(f'unknown body set {name!r} (known: {", ".join(BODY_SET_NAMES)})')

@@ -25,7 +25,7 @@ import torch
 
 from . import _lib
 from .calibration import SO101Calibration
-from .model import blob_path, read_blob, tcp_offset
+from .model import blob_path, body_set, read_blob, tcp_offset
 
 DEFAULT_CONTROL_TIMESTEP = 0.02  # task_suite.py:41
 PHYSICS_TIMESTEP = 0.002         # MuJoCo default; scene_pbr.xml sets none
@@ -448,6 +448,60 @@ class BatchedEnvironment:
     beyond 64 or raw contacts beyond 128 per substep, Jacobian blocks beyond the largest solver tier's pool).  MuJoCo has no such
     caps; counters()['contacts_dropped'] is the sum."""
     return self.debug_read('dropped').flatten().to(torch.int64)
+
+  # ------------------------------------------------------------------ contact force sensors
+  def _body_side(self, side) -> set:
+    if isinstance(side, str):
+      return set(body_set(self.model, side))
+    ids = [side] if isinstance(side, (int, np.integer)) else list(side)
+    out = set()
+    for b in ids:
+      if isinstance(b, bool) or not isinstance(b, (int, np.integer)):
+        raise ValueError(f'a body set holds body ids, a name or a list of ids, got {b!r}')
+      if not 0 <= int(b) < self.nbody:
+        raise ValueError(f'body id {int(b)} out of range (the model has {self.nbody} bodies)')
+      out.add(int(b))
+    return out
+
+  def set_contact_sensors(self, pairs):
+    """Configure up to 16 contact force sensors, one per (A, B) pair of disjoint body sets; [] turns them off (the default).  Each
+    side is a body id, an iterable of ids or a name of model.body_set for arm 0 (model.BODY_SET_NAMES); 'others' stands for every body
+    not on the other side.  After every step, contact_sensors() gives per env and sensor the net force on A from B (world
+    frame, N), the sum of the normal forces and the number of contacts, over the contacts of the step's last substep.  The
+    readout follows the new configuration from the next step on."""
+    if not self.task.collide:
+      raise ValueError('contact sensors need a task with a contact scene')
+    pairs = list(pairs)
+    if len(pairs) > _lib.MAX_CONTACT_SENSORS:
+      raise ValueError(f'at most {_lib.MAX_CONTACT_SENSORS} contact sensors, got {len(pairs)}')
+    masks = ((ctypes.c_uint32 * 2) * max(1, len(pairs)))()
+    for k, pair in enumerate(pairs):
+      if len(pair) != 2:
+        raise ValueError(f'sensor {k}: expected a pair (A, B), got {pair!r}')
+      a, b = pair
+      if isinstance(a, str) and a == 'others' and isinstance(b, str) and b == 'others':
+        raise ValueError(f"sensor {k}: only one side may be 'others'")
+      sa = None if isinstance(a, str) and a == 'others' else self._body_side(a)
+      sb = None if isinstance(b, str) and b == 'others' else self._body_side(b)
+      every = set(range(self.nbody))
+      sa = every - sb if sa is None else sa
+      sb = every - sa if sb is None else sb
+      if not sa or not sb:
+        raise ValueError(f'sensor {k}: empty body set')
+      if sa & sb:
+        raise ValueError(f'sensor {k}: bodies {sorted(sa & sb)} are on both sides')
+      masks[k][0] = sum(1 << x for x in sa); masks[k][1] = sum(1 << x for x in sb)
+    self._check(self._lib.so101_contact_sensors(self._h, len(pairs), ctypes.cast(masks, ctypes.c_void_p)))
+    self._nsensor = len(pairs)
+
+  def contact_sensors(self) -> torch.Tensor:
+    """float32 [N, K, 5] readout of the K configured sensors after the last step: net force on A from B (x, y, z; world frame,
+    newtons), sum of the normal forces, number of contacts.  Zero for envs that returned FIRST, were reset or diverged."""
+    out = torch.zeros(self.num_envs, getattr(self, '_nsensor', 0), 5, dtype=torch.float32, device=self.device)
+    if out.numel() == 0:
+      return out
+    self._check(self._lib.so101_contact_sensors_read(self._h, ctypes.c_void_p(out.data_ptr()), out.numel(), self._stream()))
+    return out
 
   KERNEL_NAMES = ("scene_begin_kernel", "scene_narrow_kernel", "scene_solve_kernel", "scene_solve_tier1_kernel", "arm_step_kernel", "scene_gjk_kernel",
                   "scene_kindyn_kernel", "scene_broad_kernel", "scene_epa_kernel", "scene_manifold_kernel", "scene_solve_tier2_kernel")
